@@ -1,6 +1,7 @@
 """EMR2A retrieval hot path benchmark (BASELINE.json metric: queries/sec, cosine Top-K + vote).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c1|c2|c2k5|c3|c4|c5|small]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload ("c2", BASELINE.json configs[1]): 1M-case database, 512-d image + 512-d text
@@ -64,13 +65,27 @@ WORKLOADS = {
 }
 C3_W_TEXT = 0.25
 Q_ROW0 = 50_003_968          # first synthetic row of the query block (far outside any database)
+DUMP_BYTES = 64 << 20        # --dump-outputs: all files together
+DUMP_QUERIES = 65536         # --dump-outputs: per-query arrays of larger workloads keep a seeded sample of this many rows
+# --dump-outputs leaves out the packed (score, index) keys, which repeat top_scores / top_idx, and the rescore arm's
+# internal status word
+NOT_DUMPED = ("keys", "status")
+
+
+def at_least(minimum):
+    def parse_count(text):
+        value = int(text)
+        if value < minimum:
+            raise argparse.ArgumentTypeError(f"must be >= {minimum}, got {value}")
+        return value
+    return parse_count
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=at_least(1), default=10, help="timed steps")
+    ap.add_argument("--warmup", type=at_least(0), default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default=os.environ.get("EMR2A_BENCH_WORKLOAD", "c2"), choices=sorted(WORKLOADS))
     ap.add_argument("--precision", default=os.environ.get("EMR2A_BENCH_PRECISION", "rescore"))
@@ -81,7 +96,42 @@ def parse():
     ap.add_argument("--shard-of", type=int, default=int(os.environ.get("EMR2A_BENCH_SHARD_OF", 1)),
                     help="profiling aid (single GPU): search only shard 0 of this many row shards, i.e. the kernel a rank of "
                          "an N-GPU run launches -- ncu cannot follow a multi-rank job; the line is marked and is not a bench value")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the arrays the last timed step returned as DIR/<name>.npy "
+                         "(see dump_outputs)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 arm; --impl reference has none to write")
+    return args
+
+
+def dump_outputs(out_dir, results, n_queries):
+    """Write what the last timed step returned to its caller as ``out_dir/<name>.npy``, so that two builds can be
+    compared output for output: the inputs are seeded, the same arguments give the same arrays.  ``results`` maps
+    names to tensors; those named in NOT_DUMPED are not written.  Floating-point arrays are written as float32
+    (float64 stays float64), integer ones as float64, which holds every index and count exactly.  When there are
+    more than DUMP_QUERIES queries, per-query arrays (first dimension ``n_queries``) keep a fixed, seeded sample of
+    DUMP_QUERIES rows; their query numbers are written as query_rows.npy."""
+    import torch
+    rows = None
+    if n_queries > DUMP_QUERIES:
+        rows = np.sort(np.random.default_rng(0).choice(n_queries, DUMP_QUERIES, replace=False))
+    arrays = {}
+    for name, t in results.items():
+        if not torch.is_tensor(t) or name in NOT_DUMPED:
+            continue
+        if rows is not None and t.dim() > 0 and t.shape[0] == n_queries:
+            t = t[torch.from_numpy(rows).to(t.device)]
+        a = t.cpu().numpy()
+        arrays[name] = a.astype(np.float32 if a.dtype.kind == "f" and a.itemsize <= 4 else np.float64)
+    if rows is not None:
+        arrays["query_rows"] = rows.astype(np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def workload_string(name, n_db=None):
@@ -330,7 +380,7 @@ def c5_rows_for(world):
     return int(round(n * (world / 8.0) ** 0.5 / 100_000.0)) * 100_000
 
 
-def c5_record(args, eng, dev, world, rank, local_rank, n, steps, warm_full, cpu_sample):
+def c5_record(args, eng, dev, world, rank, local_rank, n, steps, warm_full, cpu_sample, dump_dir=None):
     """BASELINE.json configs[4]: N-case 1024-d fused database, EVERY case a query, 5-fold CV rule (a case is never
     retrieved from its own fold), K=5.  Rows are in fold order (fold = contiguous fifths of the synthetic,
     label-shuffled rows) and sharded FOLD-BALANCED: rank r holds piece r of every fold (SURVEY 8e).  Per step and
@@ -401,6 +451,8 @@ def c5_record(args, eng, dev, world, rank, local_rank, n, steps, warm_full, cpu_
     clocks = sampler.stop(windows) if rank == 0 else None
     launches = eng.launches - l0
     peak_mem = torch.cuda.max_memory_allocated(dev)
+    if rank == 0 and dump_dir:
+        dump_outputs(dump_dir, out, n)
     rec = None
     if rank == 0:
         pk = peaks()
@@ -463,7 +515,7 @@ def run_c5(args):
     eng = get_engine(dev)
     n = int(os.environ.get("EMR2A_C5_N", WORKLOADS["c5"][0]))
     rec = c5_record(args, eng, dev, world, rank, local_rank, n, max(1, args.steps), warm_full=args.warmup > 0,
-                    cpu_sample=0 if args.no_cpu_baseline else min(args.cpu_sample, 16))
+                    cpu_sample=0 if args.no_cpu_baseline else min(args.cpu_sample, 16), dump_dir=args.dump_outputs)
     if rank == 0:
         emit(rec)
     if world > 1:
@@ -521,6 +573,9 @@ def run_c1(args):
     e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / args.steps
     launches = eng.launches - l0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {f"fold{f + 1}_{name}": t for f, r in enumerate(res) for name, t in r.items()
+                                         if name not in NOT_DUMPED}, n)
     # e2e: the public run_cv, host preprocessing (the reference's own sklearn calls)
     np.random.seed(0)
     t0 = time.perf_counter()
@@ -732,6 +787,8 @@ def main():
         tc_avg_ms = k2_avg_ms
     ms_per_step = ms_total / args.steps
     qps = n_q / (ms_per_step / 1e3)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, res, n_q)
 
     # ---- e2e: host (pinned) inputs through the public host-buffer API ----
     e2e = None

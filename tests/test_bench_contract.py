@@ -30,11 +30,62 @@ def test_reference_arm_line_small_workload():
     assert d["gpu_launches"] == 0 and "workload" in d["config"]
 
 
+def test_step_counts_and_dump_option_are_checked():
+    for args, why in ((("--steps", "0"), "must be >= 1"), (("--warmup", "-1"), "must be >= 0"),
+                      (("--dump-outputs", "out"), "--impl reference has none to write")):
+        out = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--impl", "reference", "--workload", "small",
+                              *args], capture_output=True, text=True, timeout=120, cwd=REPO)
+        assert out.returncode == 2 and why in out.stderr, (args, out.stderr[-2000:])
+
+
+def test_dump_outputs_types_sample_and_limit(tmp_path, monkeypatch):
+    """bench.dump_outputs: float32 / float64 files, integers exact, packed keys and status left out, a seeded row
+    sample (the same rows every time) once there are more queries than DUMP_QUERIES, and the size limit."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, REPO)
+    import bench
+    n = 40
+    res = {"top_idx": torch.arange(n * 3, dtype=torch.int64).reshape(n, 3) + 2 ** 40,
+           "top_scores": torch.linspace(-1, 1, n * 3).reshape(n, 3), "pred_vote": torch.arange(n, dtype=torch.int32),
+           "hit_counts": torch.tensor([[5, 7]]), "keys": torch.zeros(n, 3, dtype=torch.int64),
+           "status": torch.zeros(4, dtype=torch.int32), "precision": "rescore"}
+    bench.dump_outputs(str(tmp_path / "all"), res, n)
+    assert sorted(os.listdir(tmp_path / "all")) == ["hit_counts.npy", "pred_vote.npy", "top_idx.npy", "top_scores.npy"]
+    got = {f[:-4]: np.load(tmp_path / "all" / f) for f in os.listdir(tmp_path / "all")}
+    assert got["top_scores"].dtype == np.float32 and np.array_equal(got["top_scores"], res["top_scores"].numpy())
+    for name in ("top_idx", "pred_vote", "hit_counts"):
+        assert got[name].dtype == np.float64 and np.array_equal(got[name].astype(np.int64), res[name].numpy())
+    monkeypatch.setattr(bench, "DUMP_QUERIES", 16)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), res, n)
+    rows = np.load(tmp_path / "s1" / "query_rows.npy")
+    assert rows.shape == (16,) and np.all(np.diff(rows) > 0)
+    assert np.array_equal(rows, np.load(tmp_path / "s2" / "query_rows.npy"))
+    r = rows.astype(np.int64)
+    assert np.array_equal(np.load(tmp_path / "s1" / "top_idx.npy").astype(np.int64), res["top_idx"].numpy()[r])
+    assert np.array_equal(np.load(tmp_path / "s1" / "hit_counts.npy"), [[5, 7]])
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100)
+    with pytest.raises(RuntimeError, match="limit"):
+        bench.dump_outputs(str(tmp_path / "big"), res, n)
+    assert not os.path.exists(tmp_path / "big")
+
+
 @pytest.mark.gpu
-def test_b200_arm_line_small_workload():
-    d = _run("--workload", "small", "--steps", "3", "--warmup", "3", "--cpu-sample", "8")
+def test_b200_arm_line_small_workload(tmp_path):
+    import numpy as np
+    dump = tmp_path / "outputs"
+    d = _run("--workload", "small", "--steps", "3", "--warmup", "3", "--cpu-sample", "8", "--dump-outputs", str(dump))
     assert BASE_KEYS | {"roofline", "clocks"} <= set(d)
     assert d["n_gpus"] == 1 and d["value"] > 0 and d["gpu_launches"] > 0 and d["data"] == "synthetic"
+    assert d["steps"] == 3
+    out = {f[:-4]: np.load(dump / f) for f in os.listdir(dump)}
+    assert {"top_idx", "top_scores", "top_labels", "pred_vote", "pred_weighted", "hit_counts"} <= set(out)
+    assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    assert out["top_idx"].shape == (2048, 10) and out["top_idx"].min() >= 0 and out["top_idx"].max() < 100_000
+    assert np.all(np.diff(out["top_scores"], axis=1) <= 0)
+    assert out["hit_counts"][0, 0] / 2048 == d["accuracy"]["top1"]
     r = d["roofline"]
     assert r["bound"] == "tensor" and r["unit"] == "TFLOP/s" and abs(r["frac"] - r["achieved"] / r["peak"]) < 1e-9
     e = d["e2e"]

@@ -187,10 +187,13 @@ def test_dropin_shims_exist_for_every_reference_module():
                          "compute_precision_recall_f1", "compute_confusion_matrix"]
 
 
-REFERENCE = os.environ.get("EMR2A_REFERENCE", "/root/reference")
+# The next three tests launch the reference project's own scripts, so they need a checkout of it; the repository
+# cannot carry that tree.  tests/test_gpu_scripts_replay.py checks the same entry points against stored outputs.
+REFERENCE = os.environ.get("EMR2A_REFERENCE", "")
+NO_REFERENCE = "set EMR2A_REFERENCE to a checkout of the reference project to run its scripts on the drop-in"
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, "pipelines")), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not (REFERENCE and os.path.isdir(os.path.join(REFERENCE, "pipelines"))), reason=NO_REFERENCE)
 def test_reference_scripts_run_on_the_dropin(tmp_path):
     """The reference's own step-3 script, launched unchanged through emr2a_b200/run.py from the reference
     root, must reach THIS implementation: without a GPU it stops at our 'no CPU fallback' error instead of
@@ -223,7 +226,7 @@ def test_reference_scripts_run_on_the_dropin(tmp_path):
         assert "emr2a_b200" in out.stderr
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, "analysis")), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not (REFERENCE and os.path.isdir(os.path.join(REFERENCE, "analysis"))), reason=NO_REFERENCE)
 def test_dropin_import_resolution_from_reference_root():
     import subprocess
     import sys
@@ -297,7 +300,7 @@ def test_public_signatures_match_the_reference():
     assert checked >= 35
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, "analysis")), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not (REFERENCE and os.path.isdir(os.path.join(REFERENCE, "analysis"))), reason=NO_REFERENCE)
 def test_run_cv_experiments_script_reaches_the_dropin(tmp_path):
     """analysis/run_cv_experiments.py launched UNCHANGED through emr2a_b200/run.py from the reference root
     (--skip_encoding, the layout of :111-128): every import of the script resolves (encoders, utils.vlm_review through
