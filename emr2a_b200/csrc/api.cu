@@ -1,6 +1,7 @@
 // C-ABI glue: error text, device check, emr2a_topk_search dispatch.
 #include "common.cuh"
 
+#include <math.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -47,6 +48,11 @@ int tc_topk_search(const uint16_t* q_hi, const uint16_t* q_lo, const uint16_t* d
 int tc_planned_splits(int64_t Q, int64_t N, int min_splits);
 int tc_timing_enable(int on);
 int tc_timing_read(float* ms_out, int cap, int* n_out);
+void tc_timing_record(int which, cudaStream_t st);
+int tc_range_filter(const uint16_t* q_hi, const uint16_t* db_hi, int64_t Q, int64_t N, int D, int64_t ldq, int64_t lddb,
+                    const uint8_t* q_fold, const uint8_t* db_fold, int fold_sorted, int64_t idx_base, float min_score,
+                    const float* q_stats, const float* db_stats, uint64_t* cand, int64_t cand_cap,
+                    unsigned long long* count, void* workspace, size_t ws_bytes, cudaStream_t st);
 
 size_t rescore_workspace_bytes(int64_t Q, int K);
 int rescore_pipeline(const uint64_t* approx, int KP, const uint32_t* tau, const float* q, int64_t ldq, const float* db,
@@ -68,6 +74,11 @@ int rescore_exact_rescan(const float* q, int64_t ldq, const float* db, int64_t l
                          int n_flagged, uint64_t* out_compact, void* workspace, size_t ws_bytes, const uint16_t* db_hi,
                          int64_t lddb_hi, const float* q_stats, const float* db_stats, const uint64_t* seed_keys,
                          cudaStream_t st);
+
+int range_refine_check(const float* q, int64_t ldq, const float* db, int64_t lddb, const emr2a_lazy_rows* db_lazy, int D);
+int range_refine(const uint64_t* cand, int64_t cand_cap, unsigned long long* counts, uint64_t* out, int64_t out_cap,
+                 const float* q, int64_t ldq, const float* db, int64_t lddb, const emr2a_lazy_rows* db_lazy, int D,
+                 int64_t idx_base, float min_score, cudaStream_t st);
 
 constexpr int RESCORE_KP = 32;    // candidates kept per (query, database split) by the filter; 16 leaves too little slack (measured)
 constexpr int RESCORE_KPM = 64;   // candidates per query re-scored after merging the splits
@@ -315,7 +326,47 @@ extern "C" int emr2a_exact_rescan(const float* q_f32, int64_t ldq_f32, const flo
                               n_flagged, out_keys, workspace, ws_bytes, db_hi, lddb_bf16, q_stats, db_stats, seed_keys, st);
 }
 
+// ---- range search: every admissible pair with exact score >= min_score --------------------------------------------
+extern "C" size_t emr2a_range_search_workspace_bytes(int64_t Q, int64_t N, int D) {
+  if (Q <= 0 || N <= 0 || D <= 0) return 256;
+  return align256(tc_topk_workspace_bytes(Q, N, 1, D));
+}
+
+extern "C" int emr2a_range_search(const float* q_f32, int64_t ldq_f32, const uint16_t* q_hi, int64_t ldq_bf16,
+                                  const float* db_f32, int64_t lddb_f32, const uint16_t* db_hi, int64_t lddb_bf16,
+                                  int64_t Q, int64_t N, int D, const uint8_t* q_fold, const uint8_t* db_fold,
+                                  int fold_sorted, int64_t idx_base, float min_score, const float* q_stats,
+                                  const float* db_stats, uint64_t* cand, int64_t cand_cap, uint64_t* results,
+                                  int64_t result_cap, uint64_t* counts_out, void* workspace, size_t ws_bytes,
+                                  const emr2a_lazy_rows* db_lazy, void* stream) {
+  if (Q < 0 || N < 0 || D <= 0 || cand_cap < 0 || result_cap < 0 || !counts_out || (cand_cap > 0 && !cand) ||
+      (result_cap > 0 && !results))
+    return fail(EMR2A_ERR_INVALID, "range_search: bad arguments (Q=%lld N=%lld D=%d)", (long long)Q, (long long)N, D);
+  if (!isfinite(min_score)) return fail(EMR2A_ERR_INVALID, "range_search: min_score must be finite");
+  if ((q_fold == nullptr) != (db_fold == nullptr)) return fail(EMR2A_ERR_INVALID, "range_search: q_fold and db_fold must be given together");
+  if (idx_base < 0) return fail(EMR2A_ERR_INVALID, "range_search: negative idx_base");
+  if (!q_f32 || (!db_f32 && !db_lazy) || !q_stats || !db_stats)
+    return fail(EMR2A_ERR_INVALID, "range_search: q_f32, db_f32 (or db_lazy), q_stats and db_stats required");
+  if (ldq_f32 < D || (!db_lazy && lddb_f32 < D)) return fail(EMR2A_ERR_INVALID, "range_search: leading dimension smaller than D");
+  if (Q == 0 || N == 0) return EMR2A_OK;
+  if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) return fail(EMR2A_ERR_INVALID, "range_search: workspace must be 256-byte aligned");
+  // the refine stage's operand rules are checked before anything is launched: an error leaves the outputs untouched
+  int rc = range_refine_check(q_f32, ldq_f32, db_f32, lddb_f32, db_lazy, D);
+  if (rc != EMR2A_OK) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  unsigned long long* counts = reinterpret_cast<unsigned long long*>(counts_out);
+  rc = tc_range_filter(q_hi, db_hi, Q, N, D, ldq_bf16, lddb_bf16, q_fold, db_fold, fold_sorted, idx_base, min_score,
+                           q_stats, db_stats, cand, cand_cap, counts, workspace, ws_bytes, st);
+  if (rc != EMR2A_OK) return rc;
+  tc_timing_record(0, st);
+  rc = range_refine(cand, cand_cap, counts, results, result_cap, q_f32, ldq_f32, db_f32, lddb_f32, db_lazy, D, idx_base,
+                    min_score, st);
+  tc_timing_record(1, st);
+  return rc;
+}
+
 // Diagnostics: time the Top-K kernel of every search alone (CUDA events on the launching stream around its launch).
+// A range search (emr2a_range_search) adds two entries: its filter kernel, then its refine kernel.
 // enable != 0 starts a fresh series; emr2a_debug_tc_elapsed waits for the timed launches and returns their durations
 // (milliseconds, HOST array, oldest first, the last `cap` at most).
 extern "C" int emr2a_debug_tc_timing(int enable) { return tc_timing_enable(enable); }

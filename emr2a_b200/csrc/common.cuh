@@ -92,6 +92,17 @@ __device__ __forceinline__ uint2 ldg_stream_u2(const uint2* p) {
   return r;
 }
 
+// Bound E on |s~ - s| of the rescore arm (derivation: rescore.cu), from the query's norms nq, rq and the database's
+// K1 stats ds.  Shared by the re-scoring kernels and the range epilogue of the tensor-core filter (tc_common.cuh).
+__device__ __forceinline__ float error_bound(float nq, float rq, const float* ds, int D) {
+  // the four norms are fp32 sums of D squares (relative error of a norm <= D * 2^-25): widen them accordingly
+  const float up = 1.f + static_cast<float>(D) * 5.9604645e-8f;
+  const float nd = ds[0] * up, rd = ds[1] * up;
+  nq *= up; rq *= up;
+  const float arith = (1.02f * static_cast<float>(D) + 8.f) * 1.1920929e-7f * (nq + rq) * (nd + rd);
+  return (rq * nd + (nq + rq) * rd + arith) * 1.000001f + 1e-30f;      // rounded up: the bound must stay a bound
+}
+
 // split an fp32 value into bf16 hi + bf16 lo (2-way split, x ~= hi + lo, rel. residual ~2^-17)
 __device__ __forceinline__ void split_bf16(float x, uint16_t& hi, uint16_t& lo) {
   __nv_bfloat16 h = __float2bfloat16_rn(x);

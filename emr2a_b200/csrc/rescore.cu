@@ -76,15 +76,6 @@ __device__ __forceinline__ int flagged_count(const RescoreParams& p) {
 template <int SRC> struct RawOf { typedef float T; };
 template <> struct RawOf<2> { typedef __nv_bfloat16 T; };
 
-__device__ __forceinline__ float error_bound(float nq, float rq, const float* ds, int D) {
-  // the four norms are fp32 sums of D squares (relative error of a norm <= D * 2^-25): widen them accordingly
-  const float up = 1.f + static_cast<float>(D) * 5.9604645e-8f;
-  const float nd = ds[0] * up, rd = ds[1] * up;
-  nq *= up; rq *= up;
-  const float arith = (1.02f * static_cast<float>(D) + 8.f) * 1.1920929e-7f * (nq + rq) * (nd + rd);
-  return (rq * nd + (nq + rq) * rd + arith) * 1.000001f + 1e-30f;      // rounded up: the bound must stay a bound
-}
-
 // The query side of the bound is taken per query: ||q|| and ||q - bf16(q)|| of THIS query's fp32 row (the hi plane
 // the filter used is bf16_rn of exactly these values), clamped by the batch maxima K1 wrote.  Batches whose query
 // norms differ (late fusion with per-query z-score / min-max scaling, emr2a_b200/late.py) get a bound as tight as a
@@ -859,6 +850,101 @@ int rescore_exact_rescan(const float* q, int64_t ldq, const float* db, int64_t l
   const int rc = lazy_fill(p, db_lazy, D);
   if (rc != EMR2A_OK) return rc;
   return launch_rescan(p, rows_src(db_lazy), st);
+}
+
+// ---- range search, refine stage (emr2a_range_search) ----------------------------------------------------------------
+// The filter emitted every admissible pair with s~ >= t - E; the exact score s of each is computed here and the pair is
+// kept iff s >= t.  A warp per candidate, in the arithmetic and reduction order of rescore_select_kernel (128-bit
+// chunks, four fused multiply-adds each, then warp_sum; 32-bit chunks without the 128-bit path), so the scores are
+// bit-identical to the ones the Top-K of the rescore arm reports for the same pair.
+struct RangeRefineParams {
+  const ulonglong2* cand;                  // [min(counts[0], cand_cap)] (query, approximate key)
+  int64_t cand_cap;
+  unsigned long long* counts;              // [0] candidates (filter), [1] results (here)
+  ulonglong2* out;                         // [out_cap] (query, exact key)
+  int64_t out_cap;
+  const float* q; int64_t ldq;
+  const float* db; int64_t lddb;
+  LazyRows lazy;
+  int D;
+  int64_t idx_base;
+  float t;
+};
+
+template <bool VEC, int SRC>
+__global__ void __launch_bounds__(256) range_refine_kernel(const RangeRefineParams p) {
+  static_assert(SRC == 0 || VEC, "deferred fp32 rows need the 128-bit path");
+  const unsigned long long n = p.counts[0];
+  if (n > static_cast<unsigned long long>(p.cand_cap)) return;      // incomplete candidate list: the caller retries
+  const int lane = threadIdx.x & 31;
+  const unsigned long long warps = static_cast<unsigned long long>(gridDim.x) * (blockDim.x >> 5);
+  for (unsigned long long i = (static_cast<unsigned long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; i < n; i += warps) {
+    const ulonglong2 c = p.cand[i];
+    const uint32_t gidx = key_index(c.y);
+    const int64_t row = static_cast<int64_t>(gidx) - p.idx_base;
+    const float* qrow = p.q + static_cast<int64_t>(c.x) * p.ldq;
+    float acc = 0.f;
+    if (VEC) {
+      LazyRowCtx ctx;
+      if (SRC != 0) ctx = lazy_row_ctx(p.lazy, row);
+      for (int e = lane * 4; e < p.D; e += 128) {
+        const float4 x = __ldg(reinterpret_cast<const float4*>(qrow + e));
+        const float4 y = SRC == 0 ? __ldg(reinterpret_cast<const float4*>(p.db + row * p.lddb + e))
+                                  : lazy_load4<typename RawOf<SRC>::T>(p.lazy, ctx, row, e);
+        acc = fmaf(x.x, y.x, acc); acc = fmaf(x.y, y.y, acc);
+        acc = fmaf(x.z, y.z, acc); acc = fmaf(x.w, y.w, acc);
+      }
+    } else {
+      for (int e = lane; e < p.D; e += 32) acc = fmaf(__ldg(qrow + e), __ldg(p.db + row * p.lddb + e), acc);
+    }
+    const float s = warp_sum(acc);
+    if (lane == 0 && s >= p.t) {
+      const unsigned long long pos = atomicAdd(p.counts + 1, 1ull);
+      if (pos < static_cast<unsigned long long>(p.out_cap)) p.out[pos] = make_ulonglong2(c.x, pack_key(s, gidx));
+    }
+  }
+}
+
+template <int SRC>
+static void launch_refine_src(const RangeRefineParams& p, bool vec, unsigned blocks, cudaStream_t st) {
+  if (vec) range_refine_kernel<true, SRC><<<blocks, 256, 0, st>>>(p);
+  else if constexpr (SRC == 0) range_refine_kernel<false, 0><<<blocks, 256, 0, st>>>(p);
+}
+
+// Operand rules of the refine stage (deferred rows, 128-bit path): fills rp, launches nothing.
+static int range_refine_operands(RescoreParams& rp, const float* q, int64_t ldq, const float* db, int64_t lddb,
+                                 const emr2a_lazy_rows* db_lazy, int D) {
+  rp.q = q; rp.ldq = ldq; rp.db = db; rp.lddb = lddb; rp.D = D;
+  const int rc = lazy_fill(rp, db_lazy, D);
+  if (rc != EMR2A_OK) return rc;
+  if (rows_src(db_lazy) != 0 && !rows_vec(rp, rows_src(db_lazy)))
+    return fail(EMR2A_ERR_UNSUPPORTED, "deferred fp32 rows need 16-byte aligned fp32 query rows with D %% 4 == 0");
+  return EMR2A_OK;
+}
+
+int range_refine_check(const float* q, int64_t ldq, const float* db, int64_t lddb, const emr2a_lazy_rows* db_lazy, int D) {
+  RescoreParams rp{};
+  return range_refine_operands(rp, q, ldq, db, lddb, db_lazy, D);
+}
+
+int range_refine(const uint64_t* cand, int64_t cand_cap, unsigned long long* counts, uint64_t* out, int64_t out_cap,
+                 const float* q, int64_t ldq, const float* db, int64_t lddb, const emr2a_lazy_rows* db_lazy, int D,
+                 int64_t idx_base, float min_score, cudaStream_t st) {
+  RescoreParams rp{};
+  const int rc = range_refine_operands(rp, q, ldq, db, lddb, db_lazy, D);
+  if (rc != EMR2A_OK) return rc;
+  const int src = rows_src(db_lazy);
+  const bool vec = rows_vec(rp, src);
+  RangeRefineParams p{};
+  p.cand = reinterpret_cast<const ulonglong2*>(cand); p.cand_cap = cand_cap; p.counts = counts;
+  p.out = reinterpret_cast<ulonglong2*>(out); p.out_cap = out_cap;
+  p.q = q; p.ldq = ldq; p.db = db; p.lddb = lddb; p.lazy = rp.lazy; p.D = D; p.idx_base = idx_base; p.t = min_score;
+  const unsigned blocks = static_cast<unsigned>(8 * sm_count());      // grid-stride: the candidate count is on the device
+  if (src == 0) launch_refine_src<0>(p, vec, blocks, st);
+  else if (src == 1) launch_refine_src<1>(p, vec, blocks, st);
+  else launch_refine_src<2>(p, vec, blocks, st);
+  EMR2A_LAUNCH_CHECK("range_refine_kernel");
+  return EMR2A_OK;
 }
 
 }  // namespace emr2a

@@ -33,6 +33,14 @@ struct TcParams {
   int sync_budget;         // SM cycles a pair waits at a meeting point at most (pacing only, never required for correctness)
   uint32_t* sync_ctr;      // [cohort slots][sync_points], zeroed per launch
   unsigned long long* unit_clock;  // optional [n_units][2] globaltimer at unit start / end (diagnostics)
+  // ---- range epilogue (scan_tile RANGE mode, emr2a_range_search) ----
+  float range_t;                   // min_score t; the cut is t - E, rounded down (range_cut)
+  int D;
+  const float* q_stats;            // K1 stats of both sides: the query side's batch maxima clamp every query
+  const float* db_stats;
+  ulonglong2* range_out;           // [range_cap] (query, packed key) of every pair with s~ >= cut
+  int64_t range_cap;
+  unsigned long long* range_count; // pairs found (keeps counting past range_cap)
 };
 
 // ---- PTX wrappers -------------------------------------------------------------------
@@ -164,10 +172,54 @@ __device__ __forceinline__ bool tile_skipped(const TcParams& p, int ufold, int64
 }
 
 
+// Cut of the range epilogue: every pair with exact score s >= t has s~ >= s - E >= t - E, so emitting s~ >= cut with
+// cut <= t - E (subtraction rounded down) misses none of them.  E is error_bound with the query side's batch maxima.
+// The cut is clamped to -FLT_MAX: t - E rounds to -inf for t near -FLT_MAX (or an infinite E), and -inf is what the
+// epilogue writes for the columns past N and for fold-masked pairs -- those must never pass the inclusive compare.
+// -FLT_MAX is still a lower bound of every finite score.
+__device__ __forceinline__ float range_cut(const TcParams& p) {
+  return fmaxf(__fsub_rd(p.range_t, error_bound(__ldg(p.q_stats), __ldg(p.q_stats + 1), p.db_stats, p.D)), -3.402823466e38f);
+}
+
+// Range epilogue of one 32-column chunk: the thread emits every score of its query row with s~ >= cut.  One atomicAdd
+// per warp and chunk, only when the chunk has candidates; a lane's slots follow from the warp prefix sum of the
+// per-lane counts.  Past range_cap the counter keeps counting and nothing is written.
+__device__ __forceinline__ void range_emit(const TcParams& p, const float (&v)[32], const float cut, const int64_t c0,
+                                           const int64_t q) {
+  uint32_t mask = 0u;
+  if (q < p.Q) {
+#pragma unroll
+    for (int c = 0; c < 32; ++c) mask |= (v[c] >= cut) ? (1u << c) : 0u;
+  }
+  if (!__any_sync(0xffffffffu, mask != 0u)) return;
+  const int lane = threadIdx.x & 31;
+  const int n = __popc(mask);
+  int incl = n;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int t = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += t;
+  }
+  const int total = __shfl_sync(0xffffffffu, incl, 31);
+  unsigned long long base = 0ull;
+  if (lane == 0) base = atomicAdd(p.range_count, static_cast<unsigned long long>(total));
+  base = __shfl_sync(0xffffffffu, base, 0);
+  unsigned long long pos = base + static_cast<unsigned long long>(incl - n);
+  while (mask) {
+    const int c = __ffs(mask) - 1;
+    mask &= mask - 1u;
+    if (pos < static_cast<unsigned long long>(p.range_cap))
+      p.range_out[pos] = make_ulonglong2(static_cast<unsigned long long>(q),
+                                         pack_key(select32(v, c), static_cast<uint32_t>(c0 + c + p.idx_base)));
+    ++pos;
+  }
+}
+
 // Epilogue of one 128 x 256 accumulator tile for the thread's own query row: compare-mostly scan of
 // the 256 scores in 8 chunks of 32 TMEM columns, rare sorted insertion into the register list.
+// RANGE: no list; thr is the fixed cut of range_cut and every score >= thr is emitted (range_emit).
 //   taddr = TMEM address of (this warp's lane quarter, first column of the accumulator)
-template <int KCAP, bool HAS_FOLD>
+template <int KCAP, bool HAS_FOLD, bool RANGE = false>
 __device__ __forceinline__ void scan_tile(const TcParams& p, RegTopK<KCAP>& top, float& thr, const float thr0,
                                           const uint32_t taddr, const int64_t n0, const uint32_t my_fold,
                                           const int64_t q) {
@@ -208,20 +260,24 @@ __device__ __forceinline__ void scan_tile(const TcParams& p, RegTopK<KCAP>& top,
         v[c] = (f == my_fold) ? -INFINITY : v[c];
       }
     }
-    float mx = v[0];
+    if constexpr (RANGE) {
+      range_emit(p, v, thr, c0, q);
+    } else {
+      float mx = v[0];
 #pragma unroll
-    for (int c = 1; c < 32; ++c) mx = fmaxf(mx, v[c]);
-    if (mx > thr) {                               // rare: at least one score beats the current threshold
-      uint32_t mask = 0u;
+      for (int c = 1; c < 32; ++c) mx = fmaxf(mx, v[c]);
+      if (mx > thr) {                             // rare: at least one score beats the current threshold
+        uint32_t mask = 0u;
 #pragma unroll
-      for (int c = 0; c < 32; ++c) mask |= (v[c] > thr) ? (1u << c) : 0u;
-      while (mask) {
-        const int c = __ffs(mask) - 1;
-        mask &= mask - 1u;
-        const float val = select32(v, c);
-        if (val > thr) {
-          top.insert(val, static_cast<uint32_t>(c0 + c + p.idx_base));
-          thr = fmaxf(top.threshold(), thr0);
+        for (int c = 0; c < 32; ++c) mask |= (v[c] > thr) ? (1u << c) : 0u;
+        while (mask) {
+          const int c = __ffs(mask) - 1;
+          mask &= mask - 1u;
+          const float val = select32(v, c);
+          if (val > thr) {
+            top.insert(val, static_cast<uint32_t>(c0 + c + p.idx_base));
+            thr = fmaxf(top.threshold(), thr0);
+          }
         }
       }
     }

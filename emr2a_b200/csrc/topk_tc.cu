@@ -22,7 +22,7 @@
 
 namespace emr2a {
 
-template <int PASSES, int KCAP, bool HAS_FOLD>
+template <int PASSES, int KCAP, bool HAS_FOLD, bool RANGE = false>
 __global__ void __launch_bounds__(T_THREADS, 1)
 tc_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_constant__ CUtensorMap tm_q_lo,
                const __grid_constant__ CUtensorMap tm_db_hi, const __grid_constant__ CUtensorMap tm_db_lo,
@@ -144,14 +144,16 @@ tc_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_constan
     const int row = quarter * 32 + lane;
     int acc = 0; uint32_t acc_phase = 0;
     RegTopK<KCAP> top;
+    float cut = 0.f;
+    if constexpr (RANGE) cut = range_cut(p);
     for (int64_t u = blockIdx.x; u < n_units; u += gridDim.x) {
       const int64_t split = u / p.m_tiles, mt = u - split * p.m_tiles;
       const int64_t q = mt * T_BM + row;
       const int64_t t0 = split * p.tiles_per_split;
       const int64_t t1 = (t0 + p.tiles_per_split < p.n_tiles) ? t0 + p.tiles_per_split : p.n_tiles;
       const uint32_t my_fold = (HAS_FOLD && q < p.Q) ? p.q_fold[q] : 0xFFFFu;
-      top.reset();
-      const float thr0 = unit_start_threshold(p, q);
+      if constexpr (!RANGE) top.reset();
+      const float thr0 = RANGE ? cut : unit_start_threshold(p, q);
       float thr = thr0;
       const int ufold = HAS_FOLD ? unit_fold(p, mt) : -1;
       for (int64_t t = t0; t < t1; ++t) {
@@ -159,15 +161,15 @@ tc_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_constan
         const int64_t n0 = t * T_BN;
         mbar_wait(smem_u32(&bar_tfull[acc]), acc_phase);
         tcgen05_fence_after();
-        scan_tile<KCAP, HAS_FOLD>(p, top, thr, thr0,
-                                  tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + static_cast<uint32_t>(acc * T_BN),
-                                  n0, my_fold, q);
+        scan_tile<KCAP, HAS_FOLD, RANGE>(p, top, thr, thr0,
+                                         tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + static_cast<uint32_t>(acc * T_BN),
+                                         n0, my_fold, q);
         tcgen05_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(smem_u32(&bar_tempty[acc]));
         if (++acc == 2) { acc = 0; acc_phase ^= 1u; }
       }
-      if (q < p.Q) {
+      if (!RANGE && q < p.Q) {
         if (p.tau != nullptr && top.i[KCAP - 1] != 0xFFFFFFFFu) atomicMax(p.tau + q, order_f32(top.s[KCAP - 1]));
         uint64_t* dst = p.keys_out + (split * p.Q + q) * p.K;
 #pragma unroll
@@ -397,13 +399,13 @@ int tc_timing_read(float* ms_out, int cap, int* n_out) {
   return EMR2A_OK;
 }
 
-template <int PASSES, int KCAP, bool HAS_FOLD>
+template <int PASSES, int KCAP, bool HAS_FOLD, bool RANGE = false>
 static int tc_launch(const CUtensorMap& mq_hi, const CUtensorMap& mq_lo, const CUtensorMap& md_hi, const CUtensorMap& md_lo,
                      const TcParams& p, int grid, cudaStream_t st) {
   constexpr int PLANES = PASSES == 3 ? 2 : 1;
   constexpr int STAGES = PASSES == 3 ? 2 : 4;
   const size_t smem = static_cast<size_t>(STAGES) * PLANES * (T_A_BYTES + T_B_BYTES) + 1024;
-  auto kern = tc_topk_kernel<PASSES, KCAP, HAS_FOLD>;
+  auto kern = tc_topk_kernel<PASSES, KCAP, HAS_FOLD, RANGE>;
   EMR2A_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   kern<<<grid, T_THREADS, smem, st>>>(mq_hi, mq_lo, md_hi, md_lo, p);
   EMR2A_LAUNCH_CHECK("tc_topk_kernel");
@@ -417,6 +419,22 @@ static int tc_launch_fold(bool has_fold, const CUtensorMap& a, const CUtensorMap
                   : tc_launch<PASSES, KCAP, false>(a, b, c, d, p, grid, st);
 }
 
+// Shape rules of the bf16 planes (K1 layout) shared by the Top-K and the range filter.
+static int check_planes(const char* who, const uint16_t* q_hi, const uint16_t* q_lo, const uint16_t* db_hi,
+                        const uint16_t* db_lo, int64_t Q, int64_t N, int D, int64_t ldq, int64_t lddb, int64_t idx_base,
+                        int passes) {
+  const int64_t Dp = (static_cast<int64_t>(D) + T_BK - 1) / T_BK * T_BK;
+  if (ldq < Dp || lddb < Dp || (ldq % 8) || (lddb % 8))
+    return fail(EMR2A_ERR_UNSUPPORTED, "%s: planes need ld >= round_up(D,64) and ld %% 8 == 0 (ldq=%lld lddb=%lld D=%d)", who, (long long)ldq, (long long)lddb, D);
+  if (!q_hi || !db_hi || (passes == 3 && (!q_lo || !db_lo))) return fail(EMR2A_ERR_INVALID, "%s: missing operand plane", who);
+  auto mis = [](const void* ptr) { return (reinterpret_cast<uintptr_t>(ptr) & 15) != 0; };
+  if (mis(q_hi) || mis(db_hi) || (passes == 3 && (mis(q_lo) || mis(db_lo))))
+    return fail(EMR2A_ERR_UNSUPPORTED, "%s: operand planes must be 16-byte aligned", who);
+  if (Q >= (1LL << 31) || N >= (1LL << 31) - T_BN) return fail(EMR2A_ERR_UNSUPPORTED, "%s: Q/N too large for one call", who);
+  if (N + idx_base >= 0xFFFFFFFFLL) return fail(EMR2A_ERR_UNSUPPORTED, "%s: global index exceeds 32 bits", who);
+  return EMR2A_OK;
+}
+
 int tc_topk_search(const uint16_t* q_hi, const uint16_t* q_lo, const uint16_t* db_hi, const uint16_t* db_lo,
                    int64_t Q, int64_t N, int D, int64_t ldq, int64_t lddb,
                    const uint8_t* q_fold, const uint8_t* db_fold, int64_t idx_base, int K, int passes,
@@ -424,14 +442,10 @@ int tc_topk_search(const uint16_t* q_hi, const uint16_t* q_lo, const uint16_t* d
                    TcPartials* partials, int fold_sorted, int min_splits) {
   if (K > 32) return fail(EMR2A_ERR_UNSUPPORTED, "topk_search(bf16): K=%d > 32 (use EMR2A_PREC_FP32)", K);
   const int64_t Dp = (static_cast<int64_t>(D) + T_BK - 1) / T_BK * T_BK;
-  if (ldq < Dp || lddb < Dp || (ldq % 8) || (lddb % 8))
-    return fail(EMR2A_ERR_UNSUPPORTED, "topk_search(bf16): planes need ld >= round_up(D,64) and ld %% 8 == 0 (ldq=%lld lddb=%lld D=%d)", (long long)ldq, (long long)lddb, D);
-  if (!q_hi || !db_hi || (passes == 3 && (!q_lo || !db_lo))) return fail(EMR2A_ERR_INVALID, "topk_search(bf16): missing operand plane");
-  auto mis = [](const void* ptr) { return (reinterpret_cast<uintptr_t>(ptr) & 15) != 0; };
-  if (mis(q_hi) || mis(db_hi) || (passes == 3 && (mis(q_lo) || mis(db_lo))))
-    return fail(EMR2A_ERR_UNSUPPORTED, "topk_search(bf16): operand planes must be 16-byte aligned");
-  if (Q >= (1LL << 31) || N >= (1LL << 31) - T_BN) return fail(EMR2A_ERR_UNSUPPORTED, "topk_search(bf16): Q/N too large for one call");
-  if (N + idx_base >= 0xFFFFFFFFLL) return fail(EMR2A_ERR_UNSUPPORTED, "topk_search: global index exceeds 32 bits");
+  {
+    const int rc = check_planes("topk_search(bf16)", q_hi, q_lo, db_hi, db_lo, Q, N, D, ldq, lddb, idx_base, passes);
+    if (rc != EMR2A_OK) return rc;
+  }
   const bool has_fold = q_fold != nullptr;
   const bool pairs = use_cta_pairs(Q);
   TcPlan pl = tc_plan(Q, N, K, has_fold, pairs, min_splits, lddb > ldq ? lddb : ldq, passes == 3 ? 2 : 1);
@@ -508,6 +522,56 @@ int tc_topk_search(const uint16_t* q_hi, const uint16_t* q_lo, const uint16_t* d
   if (pl.splits > 1)
     return emr2a_topk_merge(reinterpret_cast<const uint64_t*>(ws + keys_off), pl.splits, Q, K, Q * K, K, K, out_keys, st);
   return EMR2A_OK;
+}
+
+void tc_timing_record(int which, cudaStream_t st) { tc_ev_record(which, st); }
+
+int tc2_range_dispatch(bool has_fold, const CUtensorMap& a, const CUtensorMap& b, const CUtensorMap& c,
+                       const CUtensorMap& d, const TcParams& p, int grid, cudaStream_t st);
+
+// Filter of emr2a_range_search: the 1-pass (hi plane) tensor-core GEMM of tc_topk_search with the range epilogue --
+// every admissible pair with s~ >= t - E goes to cand [cand_cap] as (query, key); *count (zeroed by the caller) counts
+// them all.  Workspace: tc_topk_workspace_bytes(Q, N, 1, D) (fold padding and cohort counters of the same plan).
+int tc_range_filter(const uint16_t* q_hi, const uint16_t* db_hi, int64_t Q, int64_t N, int D, int64_t ldq, int64_t lddb,
+                    const uint8_t* q_fold, const uint8_t* db_fold, int fold_sorted, int64_t idx_base, float min_score,
+                    const float* q_stats, const float* db_stats, uint64_t* cand, int64_t cand_cap,
+                    unsigned long long* count, void* workspace, size_t ws_bytes, cudaStream_t st) {
+  int rc = check_planes("range_search", q_hi, nullptr, db_hi, nullptr, Q, N, D, ldq, lddb, idx_base, 1);
+  if (rc != EMR2A_OK) return rc;
+  const int64_t Dp = (static_cast<int64_t>(D) + T_BK - 1) / T_BK * T_BK;
+  const bool has_fold = q_fold != nullptr;
+  const bool pairs = use_cta_pairs(Q);
+  const TcPlan pl = tc_plan(Q, N, 1, has_fold, pairs, 1, lddb > ldq ? lddb : ldq, 1);
+  const size_t sync_off = (pl.fold_bytes + 255) & ~static_cast<size_t>(255);
+  if (!workspace || ws_bytes < sync_off + pl.sync_bytes)
+    return fail(EMR2A_ERR_WORKSPACE, "range_search: workspace %zu < %zu", ws_bytes, sync_off + pl.sync_bytes);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  CUtensorMap mq, md;
+  if ((rc = make_plane_map(&mq, q_hi, Q, Dp, ldq, T_BM)) != EMR2A_OK) return rc;
+  if ((rc = make_plane_map(&md, db_hi, N, Dp, lddb, pairs ? T_BN / 2 : T_BN)) != EMR2A_OK) return rc;
+  TcParams p{};
+  p.Q = Q; p.N = N; p.k_chunks = static_cast<int>(Dp / T_BK);
+  p.m_tiles = pl.m_tiles; p.n_tiles = pl.n_tiles; p.splits = pl.splits; p.tiles_per_split = pl.tiles_per_split;
+  p.idx_base = idx_base; p.K = 1;
+  p.mg = pl.mg;
+  if (pairs && pl.sync_bytes) {
+    p.sync_tiles = pl.sync_tiles; p.sync_points = pl.sync_points; p.sync_budget = pl.sync_budget;
+    p.sync_ctr = reinterpret_cast<uint32_t*>(ws + sync_off);
+    EMR2A_CUDA_TRY(cudaMemsetAsync(p.sync_ctr, 0, pl.sync_bytes, st));
+  }
+  if (has_fold) {
+    EMR2A_CUDA_TRY(cudaMemsetAsync(ws, 0xFF, pl.fold_bytes, st));
+    EMR2A_CUDA_TRY(cudaMemcpyAsync(ws, db_fold, static_cast<size_t>(N), cudaMemcpyDeviceToDevice, st));
+    p.q_fold = q_fold; p.db_fold = ws; p.fold_sorted = fold_sorted;
+  }
+  p.range_t = min_score; p.D = D; p.q_stats = q_stats; p.db_stats = db_stats;
+  p.range_out = reinterpret_cast<ulonglong2*>(cand); p.range_cap = cand_cap; p.range_count = count;
+  tc_ev_record(0, st);
+  if (pairs) rc = tc2_range_dispatch(has_fold, mq, mq, md, md, p, pl.grid, st);
+  else rc = has_fold ? tc_launch<1, 8, true, true>(mq, mq, md, md, p, pl.grid, st)
+                     : tc_launch<1, 8, false, true>(mq, mq, md, md, p, pl.grid, st);
+  tc_ev_record(1, st);
+  return rc;
 }
 
 }  // namespace emr2a

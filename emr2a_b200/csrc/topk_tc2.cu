@@ -55,7 +55,7 @@ __device__ __forceinline__ void umma_bf16_2sm(uint32_t tmem_d, uint64_t desc_a, 
       "}\n" ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
 }
 
-template <int PASSES, int KCAP, bool HAS_FOLD>
+template <int PASSES, int KCAP, bool HAS_FOLD, bool RANGE = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(T_THREADS, 1)
 tc2_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_constant__ CUtensorMap tm_q_lo,
                 const __grid_constant__ CUtensorMap tm_db_hi, const __grid_constant__ CUtensorMap tm_db_lo,
@@ -190,6 +190,8 @@ tc2_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_consta
     const int row = quarter * 32 + lane;
     int acc = 0; uint32_t acc_phase = 0;
     RegTopK<KCAP> top;
+    float cut = 0.f;
+    if constexpr (RANGE) cut = range_cut(p);
     for (int64_t u = pair; u < n_units; u += n_pairs) {
       int64_t split, mt;
       unit_coords(p, u, split, mt);
@@ -197,8 +199,8 @@ tc2_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_consta
       const int64_t t0 = split * p.tiles_per_split;
       const int64_t t1 = (t0 + p.tiles_per_split < p.n_tiles) ? t0 + p.tiles_per_split : p.n_tiles;
       const uint32_t my_fold = (HAS_FOLD && q < p.Q) ? p.q_fold[q] : 0xFFFFu;
-      top.reset();
-      const float thr0 = unit_start_threshold(p, q);
+      if constexpr (!RANGE) top.reset();
+      const float thr0 = RANGE ? cut : unit_start_threshold(p, q);
       float thr = thr0;
       const int ufold = HAS_FOLD ? unit_fold(p, mt, T2_BM) : -1;
       for (int64_t t = t0; t < t1; ++t) {
@@ -206,9 +208,9 @@ tc2_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_consta
         const int64_t n0 = t * T_BN;
         mbar_wait(smem_u32(&bar_tfull[acc]), acc_phase);
         tcgen05_fence_after();
-        scan_tile<KCAP, HAS_FOLD>(p, top, thr, thr0,
-                                  tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + static_cast<uint32_t>(acc * T_BN),
-                                  n0, my_fold, q);
+        scan_tile<KCAP, HAS_FOLD, RANGE>(p, top, thr, thr0,
+                                         tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + static_cast<uint32_t>(acc * T_BN),
+                                         n0, my_fold, q);
         tcgen05_fence_before();
         __syncwarp();
         if (lane == 0) {
@@ -217,7 +219,7 @@ tc2_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_consta
         }
         if (++acc == 2) { acc = 0; acc_phase ^= 1u; }
       }
-      if (q < p.Q) {
+      if (!RANGE && q < p.Q) {
         if (p.tau != nullptr && top.i[KCAP - 1] != 0xFFFFFFFFu) atomicMax(p.tau + q, order_f32(top.s[KCAP - 1]));
         uint64_t* dst = p.keys_out + (split * p.Q + q) * p.K;
 #pragma unroll
@@ -241,13 +243,13 @@ tc2_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_consta
   }
 }
 
-template <int PASSES, int KCAP, bool HAS_FOLD>
+template <int PASSES, int KCAP, bool HAS_FOLD, bool RANGE = false>
 static int tc2_launch(const CUtensorMap& mq_hi, const CUtensorMap& mq_lo, const CUtensorMap& md_hi, const CUtensorMap& md_lo,
                       const TcParams& p, int grid, cudaStream_t st) {
   constexpr int PLANES = PASSES == 3 ? 2 : 1;
   constexpr int STAGES = PASSES == 3 ? 3 : 6;
   const size_t smem = static_cast<size_t>(STAGES) * PLANES * (T_A_BYTES + T2_BH_BYTES) + 1024;
-  auto kern = tc2_topk_kernel<PASSES, KCAP, HAS_FOLD>;
+  auto kern = tc2_topk_kernel<PASSES, KCAP, HAS_FOLD, RANGE>;
   EMR2A_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   kern<<<grid, T_THREADS, smem, st>>>(mq_hi, mq_lo, md_hi, md_lo, p);
   EMR2A_LAUNCH_CHECK("tc2_topk_kernel");
@@ -264,6 +266,12 @@ int tc2_dispatch(int passes, int kcap, bool has_fold, const CUtensorMap& a, cons
   EMR2A_TC2_CASE(3, 8) EMR2A_TC2_CASE(3, 16) EMR2A_TC2_CASE(3, 32)
 #undef EMR2A_TC2_CASE
   return fail(EMR2A_ERR_INVALID, "tc2_dispatch: unsupported (passes=%d, kcap=%d)", passes, kcap);
+}
+
+// range epilogue (emr2a_range_search): the 1-pass filter, no register list
+int tc2_range_dispatch(bool has_fold, const CUtensorMap& a, const CUtensorMap& b, const CUtensorMap& c,
+                       const CUtensorMap& d, const TcParams& p, int grid, cudaStream_t st) {
+  return has_fold ? tc2_launch<1, 8, true, true>(a, b, c, d, p, grid, st) : tc2_launch<1, 8, false, true>(a, b, c, d, p, grid, st);
 }
 
 }  // namespace emr2a

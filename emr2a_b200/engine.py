@@ -671,10 +671,8 @@ class Engine:
             n_folds = int(folds_t.max().item()) + 1 if n else 1
         labels_t = self.to_device(labels, torch.int32)
         mats = [self._embedding(x)[0] for x in segs if x is not None]
-        in_order = bool((folds_t[1:] >= folds_t[:-1]).all().item()) if n > 1 else True
-        perm = None
-        if not in_order:
-            perm = torch.argsort(folds_t.to(torch.int16), stable=True)
+        perm = _fold_order(folds_t)
+        if perm is not None:
             mats = [m.index_select(0, perm) for m in mats]
             labels_t = labels_t.index_select(0, perm)
             folds_t = folds_t.index_select(0, perm)
@@ -753,6 +751,106 @@ class Engine:
                 res[name] = out
         res.pop("keys", None)                                  # packed keys carry fold-order indices: not exported
         return res
+
+    # ------------------------------------------------------------ range search
+    def range_search(self, db_segs: Sequence, q_segs: Sequence, min_score: float, db_weights=(1.0, 1.0),
+                     q_weights=(1.0, 1.0), db_flags: int = native.NF_ROWNORM, q_flags: int = native.NF_ROWNORM,
+                     q_fold=None, db_fold=None, max_results: int = 1 << 26) -> Dict[str, torch.Tensor]:
+        """Every admissible database row with exact fp32 score >= ``min_score``, per query -- not a fixed K.  K1 in the
+        rescore layout (deferred database rows where ``defer_default`` says so), then ``emr2a_range_search``: the
+        tensor-core filter emits every pair within the error bound below ``min_score`` and each is re-scored exactly,
+        so the answer is exact and the scores equal the ones ``topk_search(precision="rescore")`` reports.  Weights
+        and flags are those of ``search_and_vote`` (early / concat fusion, late fusion ``none``).  ``q_fold`` /
+        ``db_fold``: the CV rule (pairs with equal fold ids are excluded).
+        Returns a CSR dict: ``offsets`` int64 [Q+1], ``idx`` int64, ``scores`` float32; query q's rows are
+        ``idx[offsets[q]:offsets[q+1]]``, by score descending, then index ascending.  More than ``max_results`` results
+        (or more than 4 x ``max_results`` filter candidates) raise ValueError before any buffer of that size is made."""
+        dim = sum(int(s.shape[1]) for s in db_segs if s is not None)
+        db = self.prepare(db_segs[0], db_segs[1] if len(db_segs) > 1 else None, db_weights[0], db_weights[1], db_flags,
+                          "rescore", defer_f32=self.defer_default(dim))
+        qs = self.prepare(q_segs[0], q_segs[1] if len(q_segs) > 1 else None, q_weights[0], q_weights[1], q_flags, "rescore")
+        fold_sorted = False
+        if (q_fold is None) != (db_fold is None):
+            raise ValueError("range_search: q_fold and db_fold must be given together")
+        if q_fold is not None:
+            q_fold = self.to_device(q_fold, torch.uint8)
+            db_fold = self.to_device(db_fold, torch.uint8)
+            fold_sorted = _non_decreasing(q_fold) and _non_decreasing(db_fold)
+        return self.range_search_prepared(qs, db, min_score, q_fold, db_fold, fold_sorted, max_results=max_results)
+
+    def range_search_prepared(self, q: Operand, db: Operand, min_score: float, q_fold=None, db_fold=None,
+                              fold_sorted: bool = False, idx_base: int = 0, max_results: int = 1 << 26
+                              ) -> Dict[str, torch.Tensor]:
+        """``range_search`` on operands prepared for the rescore arm (``prepare(..., "rescore")``).  ``fold_sorted``
+        promises non-decreasing fold vectors (whole tiles of the query's own fold are skipped); ``idx_base`` is added
+        to the database row numbers."""
+        pairs = self._range_pairs(q, db, min_score, q_fold, db_fold, fold_sorted, idx_base, max_results)
+        return csr_from_pairs(pairs, q.n)
+
+    def _range_pairs(self, q: Operand, db: Operand, min_score: float, q_fold, db_fold, fold_sorted: bool, idx_base: int,
+                     max_results: int, first_per_query: int = 32) -> torch.Tensor:
+        """The ABI call (plus at most one retry with buffers sized from the counts): int64 [n, 2] (query, key).  The
+        first call holds ``first_per_query`` results and four times as many candidates per query."""
+        if q.dim != db.dim:
+            raise ValueError(f"range_search: query dim {q.dim} != database dim {db.dim}")
+        if not np.isfinite(min_score):
+            raise ValueError(f"range_search: min_score must be finite, got {min_score}")
+        lazy_arg, _lazy_keep = _lazy_arg(db) if db.f32 is None else (None, None)
+        if q.f32 is None or (db.f32 is None and lazy_arg is None) or q.hi is None or db.hi is None or q.stats is None \
+                or db.stats is None:
+            raise ValueError("range_search needs operands prepared for the rescore arm (fp32 rows, bf16 planes, stats)")
+        Q, N, D = q.n, db.n, q.dim
+        if Q == 0 or N == 0:
+            return torch.zeros((0, 2), dtype=torch.int64, device=self.device)
+        if q_fold is not None:
+            q_fold = self.to_device(q_fold, torch.uint8)
+            db_fold = self.to_device(db_fold, torch.uint8)
+        ws_bytes = int(self.lib.emr2a_range_search_workspace_bytes(Q, N, D))
+        ws = torch.empty((ws_bytes + 256,), dtype=torch.uint8, device=self.device)
+        res_cap = min(max_results, max(1 << 16, first_per_query * Q))
+        cand_cap = 4 * res_cap
+        for attempt in range(2):
+            cand = torch.empty((cand_cap, 2), dtype=torch.int64, device=self.device)
+            out = torch.empty((res_cap, 2), dtype=torch.int64, device=self.device)
+            counts = torch.zeros((2,), dtype=torch.int64, device=self.device)
+            with torch.cuda.device(self.device):
+                native.check(self.lib.emr2a_range_search(
+                    q.f32.data_ptr(), _ld(q.f32), q.hi.data_ptr(), _ld(q.hi), native.ptr(db.f32),
+                    _ld(db.f32) if db.f32 is not None else 0, db.hi.data_ptr(), _ld(db.hi), Q, N, D,
+                    native.ptr(q_fold), native.ptr(db_fold), int(fold_sorted), int(idx_base), float(min_score),
+                    q.stats.data_ptr(), db.stats.data_ptr(), cand.data_ptr(), cand_cap, out.data_ptr(), res_cap,
+                    counts.data_ptr(), _round_up(ws.data_ptr(), 256), ws_bytes, lazy_arg, self._stream()))
+            self.launches += 2
+            n_cand, n_res = (int(x) for x in counts.cpu().tolist())      # the call's one host synchronisation
+            caps = range_retry_caps(n_cand, n_res, cand_cap, res_cap, max_results)
+            if caps is None:
+                return out[:n_res]
+            if attempt == 1:
+                raise RuntimeError(f"range_search: retry with exact buffer sizes still overflowed ({n_cand}, {n_res})")
+            cand_cap, res_cap = caps
+            del cand, out
+        raise AssertionError("unreachable")
+
+    def cross_fold_duplicates(self, segs: Sequence, folds, min_score: float, flags: int = native.NF_ROWNORM,
+                              max_results: int = 1 << 26) -> Dict[str, torch.Tensor]:
+        """Near-duplicate audit of a CV cohort: every pair of cases in DIFFERENT folds whose exact fp32 similarity
+        (rows as ``cv_search_and_vote`` prepares them) is >= ``min_score`` -- the cases that put one patient's data on
+        both sides of a split and inflate every CV number.  The cohort is searched against itself under the fold rule
+        in ``cv_search_and_vote``'s fold order (whole tiles of a query's own fold are skipped).  Returns each unordered
+        pair once: ``i`` < ``j`` (caller row numbers, int64), ``score`` float32, ``fold_i``, ``fold_j``; sorted by i,
+        then j."""
+        folds_t = self.to_device(folds, torch.uint8)
+        mats = [self._embedding(x)[0] for x in segs if x is not None]
+        perm = _fold_order(folds_t)
+        if perm is not None:
+            mats = [m.index_select(0, perm) for m in mats]
+            folds_t = folds_t.index_select(0, perm)
+        # one K1 pass with materialised fp32 rows serves both sides of the self-join
+        op = self.prepare(mats[0], mats[1] if len(mats) > 1 else None, 1.0, 1.0, flags, "rescore")
+        # every unordered pair is found from both ends: twice as many results as pairs.  An audit expects few pairs, so
+        # the first buffers hold two results per case; the retry sizes them from the exact counts if there are more.
+        pairs = self._range_pairs(op, op, min_score, folds_t, folds_t, True, 0, 2 * max_results, first_per_query=2)
+        return cross_fold_pairs(pairs, perm, folds_t)
 
     # ----------------------------------------------- host-buffer (end-to-end) path
     def search_and_vote_host(self, db_segs_host: Sequence, q_segs_host: Sequence, db_labels, q_labels,
@@ -845,6 +943,74 @@ class Engine:
         return out
 
 
+def _fold_order(folds: torch.Tensor) -> Optional[torch.Tensor]:
+    """Stable permutation that sorts the rows by fold (None if they already are): the order in which the CV search
+    skips whole tiles of a query's own fold."""
+    if _non_decreasing(folds):
+        return None
+    return torch.argsort(folds.to(torch.int16), stable=True)
+
+
+def _non_decreasing(v: torch.Tensor) -> bool:
+    return bool((v[1:] >= v[:-1]).all().item()) if int(v.shape[0]) > 1 else True
+
+
+def decode_keys(keys: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Packed keys (int64 storage, non-empty) -> (scores float32, global row indices int64), on the keys' device."""
+    o = (keys >> 32) & 0xFFFFFFFF
+    bits = torch.where(o >= 0x80000000, o - 0x80000000, 0xFFFFFFFF - o)
+    bits = torch.where(bits >= 0x80000000, bits - (1 << 32), bits)           # as a signed 32-bit pattern
+    return bits.to(torch.int32).view(torch.float32), 0xFFFFFFFF - (keys & 0xFFFFFFFF)
+
+
+def csr_from_pairs(pairs: torch.Tensor, n_queries: int) -> Dict[str, torch.Tensor]:
+    """(query, packed key) pairs int64 [n, 2], any order -> CSR by query; within a query by key descending, i.e.
+    score descending, then index ascending (the tie rule of the packed keys)."""
+    q, key = pairs[:, 0], pairs[:, 1]
+    signed = key ^ (-(1 << 63))                       # unsigned key order as signed int64 order
+    o1 = torch.argsort(signed, descending=True, stable=True)
+    o = o1[torch.argsort(q[o1], stable=True)]
+    q, key = q[o], key[o]
+    scores, idx = decode_keys(key)
+    counts = torch.bincount(q, minlength=n_queries) if q.numel() else torch.zeros(n_queries, dtype=torch.int64,
+                                                                                   device=pairs.device)
+    offsets = torch.zeros(n_queries + 1, dtype=torch.int64, device=pairs.device)
+    offsets[1:] = torch.cumsum(counts, 0)
+    return {"offsets": offsets, "idx": idx, "scores": scores}
+
+
+def range_retry_caps(n_cand: int, n_res: int, cand_cap: int, res_cap: int, max_results: int
+                     ) -> Optional[Tuple[int, int]]:
+    """Buffer sizes for the one retry of a range search (None: the outputs are complete).  The counts of
+    emr2a_range_search are exact; when the candidates overflowed nothing was re-scored and the results, a subset of
+    the candidates, are bounded by their count.  Raises ValueError instead of sizing past ``max_results`` results or
+    4 x ``max_results`` candidates."""
+    if n_cand > 4 * max_results:
+        raise ValueError(f"range_search: {n_cand} filter candidates exceed 4 x max_results = {4 * max_results}; "
+                         "raise min_score or max_results")
+    if n_cand > cand_cap:
+        return n_cand, max(1, min(n_cand, max_results))
+    if n_res > max_results:
+        raise ValueError(f"range_search: {n_res} results exceed max_results = {max_results}")
+    if n_res > res_cap:
+        return cand_cap, n_res
+    return None
+
+
+def cross_fold_pairs(pairs: torch.Tensor, perm: Optional[torch.Tensor], folds: torch.Tensor) -> Dict[str, torch.Tensor]:
+    """Self-join results (query, packed key) in fold order -> each unordered pair once, in caller row numbers:
+    i < j, score, fold_i, fold_j, sorted by (i, j).  ``perm[r]`` = caller row of fold-ordered row r (None: identity)."""
+    scores, b = decode_keys(pairs[:, 1])
+    a = pairs[:, 0]
+    fa, fb = folds[a].to(torch.int64), folds[b].to(torch.int64)
+    if perm is not None:
+        a, b = perm[a], perm[b]
+    keep = a < b
+    i, j, s, fi, fj = a[keep], b[keep], scores[keep], fa[keep], fb[keep]
+    o = torch.argsort(i * (int(folds.shape[0]) + 1) + j)
+    return {"i": i[o], "j": j[o], "score": s[o], "fold_i": fi[o], "fold_j": fj[o]}
+
+
 def plan_chunks(n_rows: int, chunk_rows: int, min_rows: int = 4096) -> List[Tuple[int, int]]:
     """Row ranges of a streamed database: full chunks, then a tail that halves down to ``min_rows`` -- the search of
     the last chunk is the one piece of compute that cannot hide behind a copy, so it should be short."""
@@ -925,6 +1091,19 @@ class DatabaseIndex:
         res = self._enqueue(q_segs, q_labels, k, q_weights, q_flags, k_list, want_lists)
         self._check_status(res)
         return res
+
+    def range_search(self, q_segs: Sequence, min_score: float, q_weights=(1.0, 1.0), q_flags: Optional[int] = None,
+                     max_results: int = 1 << 26) -> Dict[str, torch.Tensor]:
+        """``Engine.range_search`` against the resident rows: every row with exact score >= ``min_score``, as a CSR
+        dict.  Needs an index built with ``precision='rescore'`` (the filter reads its bf16 plane and stats)."""
+        op = self.operand
+        if self.precision != "rescore" or op.hi is None or op.stats is None or (op.f32 is None and op.lazy is None):
+            raise ValueError(f"range_search needs an index built with precision='rescore' (this one: {self.precision!r}); "
+                             "rebuild it with build_index(..., precision='rescore')")
+        eng = self.engine
+        qs = eng.prepare(q_segs[0], q_segs[1] if len(q_segs) > 1 else None, q_weights[0], q_weights[1],
+                         self.flags if q_flags is None else q_flags, "rescore")
+        return eng.range_search_prepared(qs, op, min_score, max_results=max_results)
 
     def capture(self, n_queries: int, k: int = 10, q_weights=(1.0, 1.0), q_flags: Optional[int] = None,
                 k_list: Sequence[int] = (1, 3, 5), want_lists: bool = True, seg_dims: Optional[Sequence[int]] = None

@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define EMR2A_ABI_VERSION 11
+#define EMR2A_ABI_VERSION 12
 
 enum emr2a_status {
   EMR2A_OK = 0,
@@ -263,6 +263,38 @@ int emr2a_exact_rescan(const float* q_f32, int64_t ldq_f32, const float* db_f32,
                        const emr2a_lazy_rows* db_lazy,
                        const uint16_t* db_hi, int64_t lddb_bf16, const float* q_stats, const float* db_stats,
                        const uint64_t* seed_keys, void* stream);
+
+/*
+ * Range search: EVERY admissible pair (q, d) with exact score s(q, d) >= min_score, not a fixed K.  Replaces the full
+ * score matrix of emr2a_scores followed by a threshold on the host (the reference's compute_cosine_similarity,
+ * retrieval/similarity.py:4-7, scores everything), and with fold vectors it is the all-pairs pass of a cross-fold
+ * near-duplicate audit of a CV cohort (the CV rule of utils/cv_evaluator.py:349-376).
+ * Exactness, in three lines:  the filter score s~ of the 1-pass tensor-core GEMM obeys |s~ - s| <= E (the error bound
+ * of EMR2A_PREC_BF16_RESCORE, from q_stats / db_stats); the filter emits every pair with s~ >= min_score - E (rounded
+ * down), a superset of the answer; every emitted pair is re-scored exactly in fp32 and kept iff s >= min_score.
+ * Operands are those of EMR2A_PREC_BF16_RESCORE in emr2a_topk_search (hi planes, fp32 rows or db_lazy, both stats);
+ * q_fold / db_fold / fold_sorted / idx_base as there.  The scores are bit-identical to the ones emr2a_topk_search
+ * reports for the same pair with EMR2A_PREC_BF16_RESCORE.
+ * Buffers (device, caller-provided):
+ *   cand [cand_cap][2]       uint64 (query, packed key of the FILTER score) -- scratch of the call;
+ *   results [result_cap][2]  uint64 (query, packed key of the EXACT score), in unspecified order;
+ *   counts_out [2]           uint64, zeroed by the caller: [0] number of filter candidates (exact, also past cand_cap),
+ *                            [1] number of results (exact, also past result_cap, whenever [0] <= cand_cap; if the
+ *                            candidates overflowed, no pair is re-scored and [1] stays 0).
+ *   Either count above its capacity means the outputs are incomplete; one retry with cand_cap >= counts_out[0] and
+ *   result_cap >= counts_out[1] (>= counts_out[0] if the candidates overflowed: results are a subset) succeeds.
+ * A non-finite min_score is EMR2A_ERR_INVALID; the plane rules of the tensor-core arms give EMR2A_ERR_UNSUPPORTED.
+ * workspace: emr2a_range_search_workspace_bytes(Q, N, D), 256-byte aligned.
+ */
+size_t emr2a_range_search_workspace_bytes(int64_t Q, int64_t N, int D);
+int emr2a_range_search(const float* q_f32, int64_t ldq_f32, const uint16_t* q_hi, int64_t ldq_bf16,
+                       const float* db_f32, int64_t lddb_f32, const uint16_t* db_hi, int64_t lddb_bf16,
+                       int64_t Q, int64_t N, int D,
+                       const uint8_t* q_fold, const uint8_t* db_fold, int fold_sorted, int64_t idx_base,
+                       float min_score, const float* q_stats, const float* db_stats,
+                       uint64_t* cand, int64_t cand_cap, uint64_t* results, int64_t result_cap,
+                       uint64_t* counts_out, void* workspace, size_t ws_bytes,
+                       const emr2a_lazy_rows* db_lazy, void* stream);
 
 /*
  * K3 -- merge `parts` partial Top-K lists per query into one.  Every input list must be sorted
