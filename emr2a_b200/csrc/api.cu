@@ -52,7 +52,8 @@ void tc_timing_record(int which, cudaStream_t st);
 int tc_range_filter(const uint16_t* q_hi, const uint16_t* db_hi, int64_t Q, int64_t N, int D, int64_t ldq, int64_t lddb,
                     const uint8_t* q_fold, const uint8_t* db_fold, int fold_sorted, int64_t idx_base, float min_score,
                     const float* q_stats, const float* db_stats, uint64_t* cand, int64_t cand_cap,
-                    unsigned long long* count, void* workspace, size_t ws_bytes, cudaStream_t st);
+                    unsigned long long* count, void* workspace, size_t ws_bytes, cudaStream_t st, bool tri,
+                    int64_t q_row0);
 
 size_t rescore_workspace_bytes(int64_t Q, int K);
 int rescore_pipeline(const uint64_t* approx, int KP, const uint32_t* tau, const float* q, int64_t ldq, const float* db,
@@ -356,7 +357,7 @@ extern "C" int emr2a_range_search(const float* q_f32, int64_t ldq_f32, const uin
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   unsigned long long* counts = reinterpret_cast<unsigned long long*>(counts_out);
   rc = tc_range_filter(q_hi, db_hi, Q, N, D, ldq_bf16, lddb_bf16, q_fold, db_fold, fold_sorted, idx_base, min_score,
-                           q_stats, db_stats, cand, cand_cap, counts, workspace, ws_bytes, st);
+                           q_stats, db_stats, cand, cand_cap, counts, workspace, ws_bytes, st, false, 0);
   if (rc != EMR2A_OK) return rc;
   tc_timing_record(0, st);
   rc = range_refine(cand, cand_cap, counts, results, result_cap, q_f32, ldq_f32, db_f32, lddb_f32, db_lazy, D, idx_base,
@@ -365,8 +366,46 @@ extern "C" int emr2a_range_search(const float* q_f32, int64_t ldq_f32, const uin
   return rc;
 }
 
+// ---- self-join: every pair i < j of one row set with exact score >= min_score ----------------------------------------
+extern "C" size_t emr2a_self_join_workspace_bytes(int64_t n, int D) {
+  return emr2a_range_search_workspace_bytes(n, n, D);      // fold padding of [0, n) and the counters of the band [0, n)
+}
+
+extern "C" int emr2a_self_join(const float* x_f32, int64_t ld_f32, const uint16_t* x_hi, int64_t ld_bf16, int64_t n, int D,
+                               int64_t q_begin, int64_t q_end, const uint8_t* fold, int fold_sorted, float min_score,
+                               const float* stats, uint64_t* cand, int64_t cand_cap, uint64_t* results,
+                               int64_t result_cap, uint64_t* counts_out, void* workspace, size_t ws_bytes, void* stream) {
+  if (n < 0 || D <= 0 || cand_cap < 0 || result_cap < 0 || !counts_out || (cand_cap > 0 && !cand) ||
+      (result_cap > 0 && !results))
+    return fail(EMR2A_ERR_INVALID, "self_join: bad arguments (n=%lld D=%d)", (long long)n, D);
+  if (q_begin < 0 || q_begin > q_end || q_end > n)
+    return fail(EMR2A_ERR_INVALID, "self_join: need 0 <= q_begin <= q_end <= n (q_begin=%lld q_end=%lld n=%lld)",
+                (long long)q_begin, (long long)q_end, (long long)n);
+  if (!isfinite(min_score)) return fail(EMR2A_ERR_INVALID, "self_join: min_score must be finite");
+  if (!x_f32 || !x_hi || !stats) return fail(EMR2A_ERR_INVALID, "self_join: x_f32, x_hi and stats required");
+  if (ld_f32 < D) return fail(EMR2A_ERR_INVALID, "self_join: leading dimension smaller than D");
+  if (q_begin == q_end) return EMR2A_OK;
+  if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) return fail(EMR2A_ERR_INVALID, "self_join: workspace must be 256-byte aligned");
+  int rc = range_refine_check(x_f32, ld_f32, x_f32, ld_f32, nullptr, D);
+  if (rc != EMR2A_OK) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  unsigned long long* counts = reinterpret_cast<unsigned long long*>(counts_out);
+  // queries [q_begin, q_end) against rows [q_begin, n): no row below q_begin is a partner j > i of these queries
+  const uint16_t* band = x_hi + q_begin * ld_bf16;
+  const uint8_t* band_fold = fold ? fold + q_begin : nullptr;
+  rc = tc_range_filter(band, band, q_end - q_begin, n - q_begin, D, ld_bf16, ld_bf16, band_fold, band_fold, fold_sorted,
+                       q_begin, min_score, stats, stats, cand, cand_cap, counts, workspace, ws_bytes, st, true, q_begin);
+  if (rc != EMR2A_OK) return rc;
+  tc_timing_record(0, st);
+  // candidates carry global rows on both sides: re-scored against the whole row set
+  rc = range_refine(cand, cand_cap, counts, results, result_cap, x_f32, ld_f32, x_f32, ld_f32, nullptr, D, 0, min_score, st);
+  tc_timing_record(1, st);
+  return rc;
+}
+
 // Diagnostics: time the Top-K kernel of every search alone (CUDA events on the launching stream around its launch).
-// A range search (emr2a_range_search) adds two entries: its filter kernel, then its refine kernel.
+// A range search (emr2a_range_search) or a self-join (emr2a_self_join) adds two entries: its filter kernel, then its
+// refine kernel.
 // enable != 0 starts a fresh series; emr2a_debug_tc_elapsed waits for the timed launches and returns their durations
 // (milliseconds, HOST array, oldest first, the last `cap` at most).
 extern "C" int emr2a_debug_tc_timing(int enable) { return tc_timing_enable(enable); }

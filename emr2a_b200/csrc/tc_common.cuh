@@ -41,6 +41,10 @@ struct TcParams {
   ulonglong2* range_out;           // [range_cap] (query, packed key) of every pair with s~ >= cut
   int64_t range_cap;
   unsigned long long* range_count; // pairs found (keeps counting past range_cap)
+  // ---- self-join (RANGE mode, emr2a_self_join): one row set, only the pairs i < j of global row numbers ----
+  int self_join;                   // 1: tri_skipped tiles are not computed, j <= i is masked on the diagonal tiles
+  int64_t q_row0;                  // global row number of query row 0 (added to the query field of every candidate)
+  int64_t db_row0;                 // global row number of database row 0
 };
 
 // ---- PTX wrappers -------------------------------------------------------------------
@@ -171,6 +175,19 @@ __device__ __forceinline__ bool tile_skipped(const TcParams& p, int ufold, int64
   return __ldg(p.db_fold + a) == ufold && __ldg(p.db_fold + b) == ufold;
 }
 
+// Self-join rule at tile granularity: when the last global row of database tile t is <= the first global row of the
+// unit's query tile (bm rows), every pair of the tile has j <= i -- no TMA, no MMA, no epilogue.  Evaluated by the three
+// warp roles like tile_skipped; always false outside the range epilogue.
+template <bool RANGE>
+__device__ __forceinline__ bool tri_skipped(const TcParams& p, int64_t mt, int bm, int64_t t) {
+  if constexpr (!RANGE) {
+    return false;
+  } else {
+    if (!p.self_join) return false;
+    const int64_t last = (t * T_BN + T_BN - 1 < p.N) ? t * T_BN + T_BN - 1 : p.N - 1;
+    return p.db_row0 + last <= p.q_row0 + mt * bm;
+  }
+}
 
 // Cut of the range epilogue: every pair with exact score s >= t has s~ >= s - E >= t - E, so emitting s~ >= cut with
 // cut <= t - E (subtraction rounded down) misses none of them.  E is error_bound with the query side's batch maxima.
@@ -209,7 +226,7 @@ __device__ __forceinline__ void range_emit(const TcParams& p, const float (&v)[3
     const int c = __ffs(mask) - 1;
     mask &= mask - 1u;
     if (pos < static_cast<unsigned long long>(p.range_cap))
-      p.range_out[pos] = make_ulonglong2(static_cast<unsigned long long>(q),
+      p.range_out[pos] = make_ulonglong2(static_cast<unsigned long long>(q + p.q_row0),
                                          pack_key(select32(v, c), static_cast<uint32_t>(c0 + c + p.idx_base)));
     ++pos;
   }
@@ -217,7 +234,8 @@ __device__ __forceinline__ void range_emit(const TcParams& p, const float (&v)[3
 
 // Epilogue of one 128 x 256 accumulator tile for the thread's own query row: compare-mostly scan of
 // the 256 scores in 8 chunks of 32 TMEM columns, rare sorted insertion into the register list.
-// RANGE: no list; thr is the fixed cut of range_cut and every score >= thr is emitted (range_emit).
+// RANGE: no list; thr is the fixed cut of range_cut and every score >= thr is emitted (range_emit); in a self-join the
+// scores with j <= i are set to -inf first.
 //   taddr = TMEM address of (this warp's lane quarter, first column of the accumulator)
 template <int KCAP, bool HAS_FOLD, bool RANGE = false>
 __device__ __forceinline__ void scan_tile(const TcParams& p, RegTopK<KCAP>& top, float& thr, const float thr0,
@@ -261,6 +279,13 @@ __device__ __forceinline__ void scan_tile(const TcParams& p, RegTopK<KCAP>& top,
       }
     }
     if constexpr (RANGE) {
+      if (p.self_join) {                          // diagonal tiles: a row is never paired with itself or an earlier row
+        const int64_t lim = p.q_row0 + q - p.db_row0 - c0;      // columns c <= lim of this chunk hold j <= i
+        if (lim >= 0) {
+#pragma unroll
+          for (int c = 0; c < 32; ++c) v[c] = (c <= lim) ? -INFINITY : v[c];
+        }
+      }
       range_emit(p, v, thr, c0, q);
     } else {
       float mx = v[0];

@@ -77,7 +77,7 @@ tc_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_constan
         const int64_t t1 = (t0 + p.tiles_per_split < p.n_tiles) ? t0 + p.tiles_per_split : p.n_tiles;
         const int ufold = HAS_FOLD ? unit_fold(p, mt) : -1;
         for (int64_t t = t0; t < t1; ++t) {
-          if (HAS_FOLD && tile_skipped(p, ufold, t)) continue;
+          if ((HAS_FOLD && tile_skipped(p, ufold, t)) || tri_skipped<RANGE>(p, mt, T_BM, t)) continue;
           const int n0 = static_cast<int>(t * T_BN);
           for (int kc = 0; kc < p.k_chunks; ++kc) {
             mbar_wait(smem_u32(&bar_empty[stage]), phase ^ 1u);
@@ -104,9 +104,10 @@ tc_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_constan
         const int64_t split = u / p.m_tiles;
         const int64_t t0 = split * p.tiles_per_split;
         const int64_t t1 = (t0 + p.tiles_per_split < p.n_tiles) ? t0 + p.tiles_per_split : p.n_tiles;
-        const int ufold = HAS_FOLD ? unit_fold(p, u - split * p.m_tiles) : -1;
+        const int64_t mt = u - split * p.m_tiles;
+        const int ufold = HAS_FOLD ? unit_fold(p, mt) : -1;
         for (int64_t t = t0; t < t1; ++t) {
-          if (HAS_FOLD && tile_skipped(p, ufold, t)) continue;
+          if ((HAS_FOLD && tile_skipped(p, ufold, t)) || tri_skipped<RANGE>(p, mt, T_BM, t)) continue;
           mbar_wait(smem_u32(&bar_tempty[acc]), acc_phase ^ 1u);
           tcgen05_fence_after();
           const uint32_t d_tmem = tmem_base + static_cast<uint32_t>(acc * T_BN);
@@ -157,7 +158,7 @@ tc_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_constan
       float thr = thr0;
       const int ufold = HAS_FOLD ? unit_fold(p, mt) : -1;
       for (int64_t t = t0; t < t1; ++t) {
-        if (HAS_FOLD && tile_skipped(p, ufold, t)) continue;
+        if ((HAS_FOLD && tile_skipped(p, ufold, t)) || tri_skipped<RANGE>(p, mt, T_BM, t)) continue;
         const int64_t n0 = t * T_BN;
         mbar_wait(smem_u32(&bar_tfull[acc]), acc_phase);
         tcgen05_fence_after();
@@ -532,19 +533,26 @@ int tc2_range_dispatch(bool has_fold, const CUtensorMap& a, const CUtensorMap& b
 // Filter of emr2a_range_search: the 1-pass (hi plane) tensor-core GEMM of tc_topk_search with the range epilogue --
 // every admissible pair with s~ >= t - E goes to cand [cand_cap] as (query, key); *count (zeroed by the caller) counts
 // them all.  Workspace: tc_topk_workspace_bytes(Q, N, 1, D) (fold padding and cohort counters of the same plan).
+// tri (emr2a_self_join): query and database rows are the rows [q_row0, ...) and [idx_base, ...) of ONE row set, only
+// pairs of global rows i < j are computed, and the query field of a candidate is the global row i.  The cohort pacing
+// of a self-join band runs when the workspace holds its counters (emr2a_self_join_workspace_bytes sizes them for the
+// whole cohort as one band; pacing never changes a result).
 int tc_range_filter(const uint16_t* q_hi, const uint16_t* db_hi, int64_t Q, int64_t N, int D, int64_t ldq, int64_t lddb,
                     const uint8_t* q_fold, const uint8_t* db_fold, int fold_sorted, int64_t idx_base, float min_score,
                     const float* q_stats, const float* db_stats, uint64_t* cand, int64_t cand_cap,
-                    unsigned long long* count, void* workspace, size_t ws_bytes, cudaStream_t st) {
-  int rc = check_planes("range_search", q_hi, nullptr, db_hi, nullptr, Q, N, D, ldq, lddb, idx_base, 1);
+                    unsigned long long* count, void* workspace, size_t ws_bytes, cudaStream_t st, bool tri,
+                    int64_t q_row0) {
+  const char* who = tri ? "self_join" : "range_search";
+  int rc = check_planes(who, q_hi, nullptr, db_hi, nullptr, Q, N, D, ldq, lddb, idx_base, 1);
   if (rc != EMR2A_OK) return rc;
   const int64_t Dp = (static_cast<int64_t>(D) + T_BK - 1) / T_BK * T_BK;
   const bool has_fold = q_fold != nullptr;
   const bool pairs = use_cta_pairs(Q);
   const TcPlan pl = tc_plan(Q, N, 1, has_fold, pairs, 1, lddb > ldq ? lddb : ldq, 1);
   const size_t sync_off = (pl.fold_bytes + 255) & ~static_cast<size_t>(255);
-  if (!workspace || ws_bytes < sync_off + pl.sync_bytes)
-    return fail(EMR2A_ERR_WORKSPACE, "range_search: workspace %zu < %zu", ws_bytes, sync_off + pl.sync_bytes);
+  const size_t need = tri ? sync_off : sync_off + pl.sync_bytes;
+  if (!workspace || ws_bytes < need) return fail(EMR2A_ERR_WORKSPACE, "%s: workspace %zu < %zu", who, ws_bytes, need);
+  const bool paced = pairs && pl.sync_bytes && ws_bytes >= sync_off + pl.sync_bytes;
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   CUtensorMap mq, md;
   if ((rc = make_plane_map(&mq, q_hi, Q, Dp, ldq, T_BM)) != EMR2A_OK) return rc;
@@ -554,10 +562,18 @@ int tc_range_filter(const uint16_t* q_hi, const uint16_t* db_hi, int64_t Q, int6
   p.m_tiles = pl.m_tiles; p.n_tiles = pl.n_tiles; p.splits = pl.splits; p.tiles_per_split = pl.tiles_per_split;
   p.idx_base = idx_base; p.K = 1;
   p.mg = pl.mg;
-  if (pairs && pl.sync_bytes) {
+  if (paced) {
     p.sync_tiles = pl.sync_tiles; p.sync_points = pl.sync_points; p.sync_budget = pl.sync_budget;
     p.sync_ctr = reinterpret_cast<uint32_t*>(ws + sync_off);
     EMR2A_CUDA_TRY(cudaMemsetAsync(p.sync_ctr, 0, pl.sync_bytes, st));
+  }
+  if (pairs && env_int("EMR2A_TC_UNIT_CLOCK", 0) && pl.m_tiles * pl.splits <= UNIT_CLOCK_MAX) {
+    void* sym = nullptr;
+    EMR2A_CUDA_TRY(cudaGetSymbolAddress(&sym, g_unit_clock));
+    p.unit_clock = static_cast<unsigned long long*>(sym);
+    const int64_t plan[8] = {pl.m_tiles, pl.n_tiles, pl.splits, pl.tiles_per_split, pl.mg, p.sync_tiles, pl.grid,
+                             pl.m_tiles * pl.splits};
+    for (int i = 0; i < 8; ++i) g_last_plan[i] = plan[i];
   }
   if (has_fold) {
     EMR2A_CUDA_TRY(cudaMemsetAsync(ws, 0xFF, pl.fold_bytes, st));
@@ -566,6 +582,7 @@ int tc_range_filter(const uint16_t* q_hi, const uint16_t* db_hi, int64_t Q, int6
   }
   p.range_t = min_score; p.D = D; p.q_stats = q_stats; p.db_stats = db_stats;
   p.range_out = reinterpret_cast<ulonglong2*>(cand); p.range_cap = cand_cap; p.range_count = count;
+  if (tri) { p.self_join = 1; p.q_row0 = q_row0; p.db_row0 = idx_base; }
   tc_ev_record(0, st);
   if (pairs) rc = tc2_range_dispatch(has_fold, mq, mq, md, md, p, pl.grid, st);
   else rc = has_fold ? tc_launch<1, 8, true, true>(mq, mq, md, md, p, pl.grid, st)

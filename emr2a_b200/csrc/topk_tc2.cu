@@ -115,7 +115,7 @@ tc2_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_consta
         if (leader && p.sync_tiles > 0) unit_cohort(p, u, n_pairs, n_units, slot, cohort);
         for (int64_t t = t0; t < t1; ++t) {
           // the leader's producer paces the pair (the peer's producer follows through the slot barriers); meeting
-          // points are counted in absolute tiles so that members that skip own-fold tiles still show up
+          // points are counted in absolute tiles so that members that skip own-fold or triangle tiles still show up
           if (leader && cohort > 1 && (t - t0) % p.sync_tiles == 0)
             cohort_sync(p, slot, static_cast<int>((t - t0) / p.sync_tiles), cohort);
           if (leader && p.unit_clock != nullptr && t == t0) {
@@ -123,7 +123,7 @@ tc2_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_consta
             asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
             p.unit_clock[2 * u] = now;
           }
-          if (HAS_FOLD && tile_skipped(p, ufold, t)) continue;
+          if ((HAS_FOLD && tile_skipped(p, ufold, t)) || tri_skipped<RANGE>(p, mt, T2_BM, t)) continue;
           const int n0 = static_cast<int>(t * T_BN + rank * 128);
           for (int kc = 0; kc < p.k_chunks; ++kc) {
             mbar_wait(smem_u32(&bar_empty[stage]), phase ^ 1u);
@@ -153,7 +153,7 @@ tc2_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_consta
         const int64_t t1 = (t0 + p.tiles_per_split < p.n_tiles) ? t0 + p.tiles_per_split : p.n_tiles;
         const int ufold = HAS_FOLD ? unit_fold(p, mt, T2_BM) : -1;
         for (int64_t t = t0; t < t1; ++t) {
-          if (HAS_FOLD && tile_skipped(p, ufold, t)) continue;
+          if ((HAS_FOLD && tile_skipped(p, ufold, t)) || tri_skipped<RANGE>(p, mt, T2_BM, t)) continue;
           mbar_wait(smem_u32(&bar_tempty[acc]), acc_phase ^ 1u);
           tcgen05_fence_after();
           const uint32_t d_tmem = tmem_base + static_cast<uint32_t>(acc * T_BN);
@@ -204,7 +204,7 @@ tc2_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_consta
       float thr = thr0;
       const int ufold = HAS_FOLD ? unit_fold(p, mt, T2_BM) : -1;
       for (int64_t t = t0; t < t1; ++t) {
-        if (HAS_FOLD && tile_skipped(p, ufold, t)) continue;
+        if ((HAS_FOLD && tile_skipped(p, ufold, t)) || tri_skipped<RANGE>(p, mt, T2_BM, t)) continue;
         const int64_t n0 = t * T_BN;
         mbar_wait(smem_u32(&bar_tfull[acc]), acc_phase);
         tcgen05_fence_after();

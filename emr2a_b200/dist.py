@@ -7,6 +7,8 @@ every arm returns exact fp32 scores, so results are bit-identical for any GPU co
                                   Top-K, ONE all-gather of exact keys + bounds, verification of the merged lists.
 * ``sharded_cv_search_and_vote``  every case a query (5-fold CV rule) over fold-balanced shards; query blocks of prepared
                                   rows are broadcast from their owner over NVLink, double-buffered.
+* ``self_join_ranges``             query bands of the multi-GPU self-join (``Engine.near_duplicates``): equal
+                                  admissible tensor-core tiles per rank under the triangle and fold skips.
 * host-resident databases         ``spread_device`` (ranks spread over the host bridges), ``h2d_rates`` +
                                   ``weighted_ranges`` (shards sized by each rank's host link), ``gather_host_rows``
                                   (replicated query rows copied once per node, all-gathered over NVLink).
@@ -16,6 +18,7 @@ from __future__ import annotations
 import os
 from typing import Dict, List, Optional, Sequence, Tuple
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -250,6 +253,35 @@ def fold_balanced_ranges(fold_counts: Sequence[int], rank: int, world: int, alig
         out.append((start + lo, hi - lo))
         start += n_f
     return out
+
+
+def self_join_ranges(n_rows: int, fold_counts: Optional[Sequence[int]], world: int, tile: int = 256
+                     ) -> List[Tuple[int, int]]:
+    """Query bands [q0, q1) of the ranks in a multi-GPU self-join (``Engine.near_duplicates``) of ``n_rows`` rows,
+    fold-ordered with ``fold_counts`` rows per fold (None: no folds).  The bands cover [0, n_rows), are cut at
+    ``tile``-row boundaries and hold equal numbers of ADMISSIBLE tiles, counted as the tensor-core filter counts them
+    with ``tile``-row query and database tiles: database tile b is computed for query tile a iff b >= a (triangle) and
+    not both tiles lie inside the same fold.  A band of early rows is short, one of late rows long.  Ranks past the
+    number of tiles get empty bands."""
+    n_t = (n_rows + tile - 1) // tile
+    if n_t == 0:
+        return [(0, 0)] * world
+    a = np.arange(n_t, dtype=np.int64)
+    cost = (n_t - a).astype(np.float64)                       # database tiles b >= a
+    if fold_counts is not None:
+        ends = np.cumsum(np.asarray([int(c) for c in fold_counts], dtype=np.int64))
+        first, last = a * tile, np.minimum(a * tile + tile, n_rows) - 1
+        f_lo = np.searchsorted(ends, first, side="right")      # fold of a tile's first / last row
+        f_hi = np.searchsorted(ends, last, side="right")
+        single = f_lo == f_hi
+        # single-fold tiles of one fold are consecutive: those at or after tile a are skipped for a single-fold tile a
+        for f in np.unique(f_lo[single]):
+            idx = np.nonzero(single & (f_lo == f))[0]
+            cost[idx] -= len(idx) - np.arange(len(idx))
+    cum = np.concatenate([[0.0], np.cumsum(cost)])
+    cuts = [0] + [int(np.searchsorted(cum, cum[-1] * r / world, side="left")) for r in range(1, world)] + [n_t]
+    cuts = np.maximum.accumulate(np.minimum(cuts, n_t))
+    return [(min(int(cuts[r]) * tile, n_rows), min(int(cuts[r + 1]) * tile, n_rows)) for r in range(world)]
 
 
 def ranges_to_rows(ranges: Sequence[Tuple[int, int]], device) -> torch.Tensor:

@@ -807,50 +807,144 @@ class Engine:
             db_fold = self.to_device(db_fold, torch.uint8)
         ws_bytes = int(self.lib.emr2a_range_search_workspace_bytes(Q, N, D))
         ws = torch.empty((ws_bytes + 256,), dtype=torch.uint8, device=self.device)
-        res_cap = min(max_results, max(1 << 16, first_per_query * Q))
+
+        def call(cand, cand_cap, out, res_cap, counts):
+            return self.lib.emr2a_range_search(
+                q.f32.data_ptr(), _ld(q.f32), q.hi.data_ptr(), _ld(q.hi), native.ptr(db.f32),
+                _ld(db.f32) if db.f32 is not None else 0, db.hi.data_ptr(), _ld(db.hi), Q, N, D,
+                native.ptr(q_fold), native.ptr(db_fold), int(fold_sorted), int(idx_base), float(min_score),
+                q.stats.data_ptr(), db.stats.data_ptr(), cand.data_ptr(), cand_cap, out.data_ptr(), res_cap,
+                counts.data_ptr(), _round_up(ws.data_ptr(), 256), ws_bytes, lazy_arg, self._stream())
+        return self._pairs_with_retry(call, min(max_results, max(1 << 16, first_per_query * Q)), max_results,
+                                      "range_search")
+
+    def _pairs_with_retry(self, call, res_cap: int, max_results: int, who: str) -> torch.Tensor:
+        """Run a range-type ABI call (emr2a_range_search / emr2a_self_join) with ``res_cap`` results and four times as
+        many candidates, plus at most one retry with buffers sized from the exact counts: int64 [n, 2] (query, key)."""
         cand_cap = 4 * res_cap
         for attempt in range(2):
             cand = torch.empty((cand_cap, 2), dtype=torch.int64, device=self.device)
             out = torch.empty((res_cap, 2), dtype=torch.int64, device=self.device)
             counts = torch.zeros((2,), dtype=torch.int64, device=self.device)
             with torch.cuda.device(self.device):
-                native.check(self.lib.emr2a_range_search(
-                    q.f32.data_ptr(), _ld(q.f32), q.hi.data_ptr(), _ld(q.hi), native.ptr(db.f32),
-                    _ld(db.f32) if db.f32 is not None else 0, db.hi.data_ptr(), _ld(db.hi), Q, N, D,
-                    native.ptr(q_fold), native.ptr(db_fold), int(fold_sorted), int(idx_base), float(min_score),
-                    q.stats.data_ptr(), db.stats.data_ptr(), cand.data_ptr(), cand_cap, out.data_ptr(), res_cap,
-                    counts.data_ptr(), _round_up(ws.data_ptr(), 256), ws_bytes, lazy_arg, self._stream()))
+                native.check(call(cand, cand_cap, out, res_cap, counts))
             self.launches += 2
             n_cand, n_res = (int(x) for x in counts.cpu().tolist())      # the call's one host synchronisation
             caps = range_retry_caps(n_cand, n_res, cand_cap, res_cap, max_results)
             if caps is None:
                 return out[:n_res]
             if attempt == 1:
-                raise RuntimeError(f"range_search: retry with exact buffer sizes still overflowed ({n_cand}, {n_res})")
+                raise RuntimeError(f"{who}: retry with exact buffer sizes still overflowed ({n_cand}, {n_res})")
             cand_cap, res_cap = caps
             del cand, out
         raise AssertionError("unreachable")
 
     def cross_fold_duplicates(self, segs: Sequence, folds, min_score: float, flags: int = native.NF_ROWNORM,
-                              max_results: int = 1 << 26) -> Dict[str, torch.Tensor]:
+                              max_results: int = 1 << 26, distributed: bool = False) -> Dict[str, torch.Tensor]:
         """Near-duplicate audit of a CV cohort: every pair of cases in DIFFERENT folds whose exact fp32 similarity
         (rows as ``cv_search_and_vote`` prepares them) is >= ``min_score`` -- the cases that put one patient's data on
-        both sides of a split and inflate every CV number.  The cohort is searched against itself under the fold rule
-        in ``cv_search_and_vote``'s fold order (whole tiles of a query's own fold are skipped).  Returns each unordered
+        both sides of a split and inflate every CV number.  ``near_duplicates`` with ``folds``: returns each unordered
         pair once: ``i`` < ``j`` (caller row numbers, int64), ``score`` float32, ``fold_i``, ``fold_j``; sorted by i,
         then j."""
-        folds_t = self.to_device(folds, torch.uint8)
+        return self.near_duplicates(segs, min_score, folds, flags, max_results, distributed)
+
+    def near_duplicates(self, segs: Sequence, min_score: float, folds=None, flags: int = native.NF_ROWNORM,
+                        max_results: int = 1 << 26, distributed: bool = False) -> Dict[str, torch.Tensor]:
+        """Every pair of rows i < j of one cohort whose exact fp32 similarity is >= ``min_score``, each pair once and no
+        row with itself -- whole-cohort deduplication.  Rows are prepared as ``cv_search_and_vote`` prepares them (one K1
+        pass in the rescore layout with fp32 rows); ``emr2a_self_join`` computes only the upper triangle on the tensor
+        cores and re-scores every candidate exactly, so the scores equal the ones ``range_search`` reports.  With
+        ``folds`` only pairs of different folds count, and the rows are brought into fold order so that whole tiles of
+        one fold are skipped.
+        Returns ``i`` < ``j`` (caller row numbers, int64), ``score`` float32 and, with folds, ``fold_i`` / ``fold_j``
+        (int64); sorted by i, then j.  More than ``max_results`` pairs (or more than 4 x ``max_results`` filter
+        candidates on a GPU) raise ValueError.
+        ``distributed=True``: under ``torchrun`` with an NCCL process group, every rank called with the same arrays
+        (verified with checksums): each rank prepares the whole cohort, joins its band of query rows
+        (``dist.self_join_ranges``, equal tensor-core work per rank) and the pair lists are all-gathered; every rank
+        returns the same result, bit for bit equal to ``distributed=False``."""
+        if not np.isfinite(min_score):
+            raise ValueError(f"near_duplicates: min_score must be finite, got {min_score}")
         mats = [self._embedding(x)[0] for x in segs if x is not None]
-        perm = _fold_order(folds_t)
-        if perm is not None:
-            mats = [m.index_select(0, perm) for m in mats]
-            folds_t = folds_t.index_select(0, perm)
-        # one K1 pass with materialised fp32 rows serves both sides of the self-join
+        n = int(mats[0].shape[0])
+        folds_t, perm = None, None
+        if folds is not None:
+            folds_t = self.to_device(folds, torch.uint8)
+            if int(folds_t.shape[0]) != n:
+                raise ValueError(f"near_duplicates: {int(folds_t.shape[0])} fold ids for {n} rows")
+            perm = _fold_order(folds_t)
+            if perm is not None:
+                mats = [m.index_select(0, perm) for m in mats]
+                folds_t = folds_t.index_select(0, perm)
+        q0, q1, world = 0, n, 1
+        if distributed:
+            import torch.distributed as tdist
+            from .dist import self_join_ranges
+            world, rank = tdist.get_world_size(), tdist.get_rank()
+            # cheap guard against ranks that were handed different cohorts
+            sample = torch.arange(0, n, max(1, n // 61), device=self.device)[:64]
+            sig = torch.stack([torch.tensor(float(n), device=self.device, dtype=torch.float64),
+                               torch.tensor(float(sum(int(m.shape[1]) for m in mats)), device=self.device,
+                                            dtype=torch.float64),
+                               folds_t.double().sum() if folds_t is not None else torch.zeros((), device=self.device,
+                                                                                              dtype=torch.float64)]
+                              + [m.index_select(0, sample).double().sum() for m in mats])
+            lo_sig, hi_sig = sig.clone(), sig.clone()
+            tdist.all_reduce(lo_sig, op=tdist.ReduceOp.MIN)
+            tdist.all_reduce(hi_sig, op=tdist.ReduceOp.MAX)
+            if not torch.equal(lo_sig, hi_sig):
+                raise ValueError("near_duplicates(distributed=True): the ranks were called with different cohorts "
+                                 "(row count / dim / fold / row-sample checksums differ); every rank must pass the same "
+                                 "arrays")
+            counts = None if folds_t is None else torch.bincount(folds_t.long()).cpu().tolist()
+            q0, q1 = self_join_ranges(n, counts, world)[rank]
         op = self.prepare(mats[0], mats[1] if len(mats) > 1 else None, 1.0, 1.0, flags, "rescore")
-        # every unordered pair is found from both ends: twice as many results as pairs.  An audit expects few pairs, so
-        # the first buffers hold two results per case; the retry sizes them from the exact counts if there are more.
-        pairs = self._range_pairs(op, op, min_score, folds_t, folds_t, True, 0, 2 * max_results, first_per_query=2)
-        return cross_fold_pairs(pairs, perm, folds_t)
+        if world == 1:
+            pairs = self.self_join_prepared(op, min_score, folds_t, q0, q1, max_results)
+        else:
+            from .dist import _gather_varlen
+            err, pairs = None, torch.zeros((0, 2), dtype=torch.int64, device=self.device)
+            try:
+                pairs = self.self_join_prepared(op, min_score, folds_t, q0, q1, max_results)
+            except ValueError as e:             # every rank must take the same branch: the collectives below must match
+                err = e
+            failed = torch.tensor([0 if err is None else 1], dtype=torch.int64, device=self.device)
+            tdist.all_reduce(failed, op=tdist.ReduceOp.MAX)
+            if int(failed.item()):
+                raise err if err is not None else ValueError("near_duplicates: another rank's band exceeded max_results")
+            pairs = torch.cat(_gather_varlen(pairs, world))
+            if int(pairs.shape[0]) > max_results:
+                raise ValueError(f"near_duplicates: {int(pairs.shape[0])} pairs exceed max_results = {max_results}")
+        return self_join_result(pairs, perm, folds_t, n)
+
+    def self_join_prepared(self, op: Operand, min_score: float, folds=None, q_begin: int = 0, q_end: Optional[int] = None,
+                           max_results: int = 1 << 26) -> torch.Tensor:
+        """``emr2a_self_join`` on an operand prepared for the rescore arm with fp32 rows: the pairs i < j with
+        q_begin <= i < q_end, fold[i] != fold[j] (``folds``, in the operand's row order), exact score >= min_score.
+        Returns int64 [m, 2] (i, packed key of the exact score and j), in no particular order.  The first buffers hold
+        one result per query row (the triangle finds each pair once) and the retry sizes them from the exact counts."""
+        if op.f32 is None or op.hi is None or op.stats is None:
+            raise ValueError("self_join needs an operand prepared for the rescore arm with fp32 rows (bf16 plane, stats)")
+        n, D = op.n, op.dim
+        q_end = n if q_end is None else int(q_end)
+        q_begin = int(q_begin)
+        if not 0 <= q_begin <= q_end <= n:
+            raise ValueError(f"self_join: need 0 <= q_begin <= q_end <= n, got {q_begin}, {q_end}, {n}")
+        if q_begin == q_end:
+            return torch.zeros((0, 2), dtype=torch.int64, device=self.device)
+        fold_sorted = False
+        if folds is not None:
+            folds = self.to_device(folds, torch.uint8)
+            fold_sorted = _non_decreasing(folds)
+        ws_bytes = int(self.lib.emr2a_self_join_workspace_bytes(n, D))
+        ws = torch.empty((ws_bytes + 256,), dtype=torch.uint8, device=self.device)
+
+        def call(cand, cand_cap, out, res_cap, counts):
+            return self.lib.emr2a_self_join(
+                op.f32.data_ptr(), _ld(op.f32), op.hi.data_ptr(), _ld(op.hi), n, D, q_begin, q_end, native.ptr(folds),
+                int(fold_sorted), float(min_score), op.stats.data_ptr(), cand.data_ptr(), cand_cap, out.data_ptr(),
+                res_cap, counts.data_ptr(), _round_up(ws.data_ptr(), 256), ws_bytes, self._stream())
+        return self._pairs_with_retry(call, min(max_results, max(1 << 16, q_end - q_begin)), max_results, "self_join")
 
     # ----------------------------------------------- host-buffer (end-to-end) path
     def search_and_vote_host(self, db_segs_host: Sequence, q_segs_host: Sequence, db_labels, q_labels,
@@ -1009,6 +1103,28 @@ def cross_fold_pairs(pairs: torch.Tensor, perm: Optional[torch.Tensor], folds: t
     i, j, s, fi, fj = a[keep], b[keep], scores[keep], fa[keep], fb[keep]
     o = torch.argsort(i * (int(folds.shape[0]) + 1) + j)
     return {"i": i[o], "j": j[o], "score": s[o], "fold_i": fi[o], "fold_j": fj[o]}
+
+
+def self_join_result(pairs: torch.Tensor, perm: Optional[torch.Tensor], folds: Optional[torch.Tensor], n: int
+                     ) -> Dict[str, torch.Tensor]:
+    """Self-join results (i, packed key of j) with i < j in the joined row order -> caller row numbers.  ``perm[r]`` =
+    caller row of joined row r (None: identity); a < b does not imply perm[a] < perm[b], so every pair is normalised to
+    (min, max).  Returns i < j, score, and fold_i / fold_j (of caller rows i and j) when ``folds`` (joined order) is
+    given; sorted by (i, j)."""
+    scores, b = decode_keys(pairs[:, 1])
+    a = pairs[:, 0]
+    res: Dict[str, torch.Tensor] = {}
+    if folds is not None:
+        fa, fb = folds[a].to(torch.int64), folds[b].to(torch.int64)
+    if perm is not None:
+        a, b = perm[a], perm[b]
+    swap = a > b
+    i, j = torch.where(swap, b, a), torch.where(swap, a, b)
+    o = torch.argsort(i * (int(n) + 1) + j)
+    res["i"], res["j"], res["score"] = i[o], j[o], scores[o]
+    if folds is not None:
+        res["fold_i"], res["fold_j"] = torch.where(swap, fb, fa)[o], torch.where(swap, fa, fb)[o]
+    return res
 
 
 def plan_chunks(n_rows: int, chunk_rows: int, min_rows: int = 4096) -> List[Tuple[int, int]]:

@@ -18,7 +18,7 @@ F32, BF16 = 0, 1
 NF_SEGNORM, NF_ROWNORM, NF_ZERO_GUARD, NF_STANDARDIZE = 1, 2, 4, 8
 PREC_FP32, PREC_BF16X3, PREC_BF16X1, PREC_BF16_RESCORE = 0, 1, 2, 3
 SCORE_NONE, SCORE_ZSCORE, SCORE_MINMAX = 0, 1, 2
-ABI_VERSION = 12
+ABI_VERSION = 13
 
 _p = C.c_void_p
 _i64 = C.c_int64
@@ -49,6 +49,9 @@ _SIGNATURES = {
     "emr2a_range_search_workspace_bytes": (_sz, [_i64, _i64, _int]),
     "emr2a_range_search": (_int, [_p, _i64, _p, _i64, _p, _i64, _p, _i64, _i64, _i64, _int, _p, _p, _int, _i64, _f, _p, _p,
                                   _p, _i64, _p, _i64, _p, _p, _sz, _p, _p]),
+    "emr2a_self_join_workspace_bytes": (_sz, [_i64, _int]),
+    "emr2a_self_join": (_int, [_p, _i64, _p, _i64, _i64, _int, _i64, _i64, _p, _int, _f, _p, _p, _i64, _p, _i64, _p, _p,
+                               _sz, _p]),
     "emr2a_topk_merge": (_int, [_p, _int, _i64, _int, _i64, _i64, _int, _p, _p]),
     "emr2a_keys_map_rows": (_int, [_p, _i64, _p, _i64, _i64, _p]),
     "emr2a_vote_metrics": (_int, [_p, _i64, _int, _p, _i64, _p, _p, _int, _int, C.POINTER(C.c_int32), _int, _int,

@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define EMR2A_ABI_VERSION 12
+#define EMR2A_ABI_VERSION 13
 
 enum emr2a_status {
   EMR2A_OK = 0,
@@ -295,6 +295,34 @@ int emr2a_range_search(const float* q_f32, int64_t ldq_f32, const uint16_t* q_hi
                        uint64_t* cand, int64_t cand_cap, uint64_t* results, int64_t result_cap,
                        uint64_t* counts_out, void* workspace, size_t ws_bytes,
                        const emr2a_lazy_rows* db_lazy, void* stream);
+
+/*
+ * Self-join: EVERY pair i < j of ONE row set x [n] with exact score s(i, j) >= min_score, each pair once -- the
+ * near-duplicate pairs of a cohort (the reference scores all pairs with compute_cosine_similarity,
+ * retrieval/similarity.py:4-7) and, with a fold vector, the cross-fold pairs of a CV cohort (the CV rule of
+ * utils/cv_evaluator.py:349-376).  A call covers the query band [q_begin, q_end): every pair with q_begin <= i < q_end,
+ * i < j < n, fold[i] != fold[j] when fold is given, and s >= min_score.  Bands that partition [0, n) give each pair
+ * exactly once in total (the multi-GPU audit runs one band per GPU).
+ * Exactness, in three lines:  the filter score s~ of the 1-pass tensor-core GEMM obeys |s~ - s| <= E (the error bound
+ * of EMR2A_PREC_BF16_RESCORE, from stats); the filter emits every pair i < j with s~ >= min_score - E (rounded down), a
+ * superset of the answer; every emitted pair is re-scored exactly in fp32 and kept iff s >= min_score.
+ * Only the upper triangle is computed: 256-row tiles with every j <= i are skipped, and on the tiles the diagonal
+ * crosses the scores with j <= i are masked (also for identical rows), so a row is never paired with itself.
+ * Operands: one row set as K1 writes it for EMR2A_PREC_BF16_RESCORE: fp32 rows x_f32 [n][ld_f32], the hi plane x_hi
+ * [n][ld_bf16] and its stats[2].  fold [n] (optional) and fold_sorted as in emr2a_range_search.
+ * Results: (i, packed key of the EXACT score and j) in global row numbers; the scores are bit-identical to the ones
+ * emr2a_range_search reports for the pair (i, j) with x as both operands.
+ * Buffers, counts_out[2] and the one-retry rule: as emr2a_range_search.
+ * Errors (before anything is launched; the outputs stay untouched): EMR2A_ERR_INVALID unless 0 <= q_begin <= q_end <= n,
+ * for a non-finite min_score, missing rows / plane / stats, ld_f32 < D or a workspace that is not 256-byte aligned; the
+ * plane rules of the tensor-core arms give EMR2A_ERR_UNSUPPORTED.
+ * workspace: emr2a_self_join_workspace_bytes(n, D) is enough for any band of the row set; 256-byte aligned.
+ */
+size_t emr2a_self_join_workspace_bytes(int64_t n, int D);
+int emr2a_self_join(const float* x_f32, int64_t ld_f32, const uint16_t* x_hi, int64_t ld_bf16, int64_t n, int D,
+                    int64_t q_begin, int64_t q_end, const uint8_t* fold, int fold_sorted, float min_score,
+                    const float* stats, uint64_t* cand, int64_t cand_cap, uint64_t* results, int64_t result_cap,
+                    uint64_t* counts_out, void* workspace, size_t ws_bytes, void* stream);
 
 /*
  * K3 -- merge `parts` partial Top-K lists per query into one.  Every input list must be sorted

@@ -95,5 +95,17 @@ for prec in ("rescore", "bf16x3"):
     same = all(torch.equal(auto[key], single[key]) for key in names)
     print(f"rank {rank}/{world} cv {prec}: engine auto-distributed == single-GPU: {same}", flush=True)
     ok = ok and same
+# the multi-GPU near-duplicate self-join: each rank joins its band of query rows, pair lists all-gathered
+n_sj = 120_000
+xs, _ = synth.device_block(0, n_sj, d, c, 23, dev)
+xs[n_sj // 2:n_sj // 2 + 500] = xs[:500] + 1e-3 * xs[500:1000]          # planted near-duplicates across the cohort
+sj_folds = ((torch.arange(n_sj, device=dev, dtype=torch.int64) * 7919) % 5).to(torch.uint8)
+for name, f in (("no folds", None), ("unsorted folds", sj_folds)):
+    a = eng.near_duplicates([xs], 0.999, folds=f, distributed=True)
+    b = eng.near_duplicates([xs], 0.999, folds=f, distributed=False)
+    same = set(a) == set(b) and all(torch.equal(a[key], b[key]) for key in a)
+    print(f"rank {rank}/{world} near_duplicates {name}: distributed == single-GPU: {same} ({int(b['i'].numel())} pairs)",
+          flush=True)
+    ok = ok and same and int(b["i"].numel()) > 0
 dist.barrier(); dist.destroy_process_group()
 sys.exit(0 if ok else 1)
