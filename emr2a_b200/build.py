@@ -17,7 +17,8 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 OUT = os.path.join(PKG, "libemr2a.so")
 OBJ = os.path.join(PKG, "build")
-SOURCES = ["api.cu", "normalize_fuse.cu", "simt_paths.cu", "merge_vote.cu", "topk_tc.cu", "topk_tc2.cu", "rescore.cu", "preprocess.cu", "late_fusion.cu"]
+SOURCES = ["api.cu", "normalize_fuse.cu", "simt_paths.cu", "merge_vote.cu", "topk_tc.cu", "topk_tc2.cu", "rescore.cu", "preprocess.cu", "late_fusion.cu",
+           "components.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -7,8 +7,9 @@ every arm returns exact fp32 scores, so results are bit-identical for any GPU co
                                   Top-K, ONE all-gather of exact keys + bounds, verification of the merged lists.
 * ``sharded_cv_search_and_vote``  every case a query (5-fold CV rule) over fold-balanced shards; query blocks of prepared
                                   rows are broadcast from their owner over NVLink, double-buffered.
-* ``self_join_ranges``             query bands of the multi-GPU self-join (``Engine.near_duplicates``): equal
-                                  admissible tensor-core tiles per rank under the triangle and fold skips.
+* ``self_join_ranges``             query bands of the multi-GPU self-join (``Engine.near_duplicates``,
+                                  ``Engine.duplicate_groups``): equal admissible tensor-core tiles per rank under the
+                                  triangle and fold skips; also the sub-bands of a band whose pairs overflow.
 * host-resident databases         ``spread_device`` (ranks spread over the host bridges), ``h2d_rates`` +
                                   ``weighted_ranges`` (shards sized by each rank's host link), ``gather_host_rows``
                                   (replicated query rows copied once per node, all-gathered over NVLink).
@@ -255,17 +256,24 @@ def fold_balanced_ranges(fold_counts: Sequence[int], rank: int, world: int, alig
     return out
 
 
-def self_join_ranges(n_rows: int, fold_counts: Optional[Sequence[int]], world: int, tile: int = 256
-                     ) -> List[Tuple[int, int]]:
+def self_join_ranges(n_rows: int, fold_counts: Optional[Sequence[int]], world: int, tile: int = 256,
+                     q_begin: int = 0, q_end: Optional[int] = None) -> List[Tuple[int, int]]:
     """Query bands [q0, q1) of the ranks in a multi-GPU self-join (``Engine.near_duplicates``) of ``n_rows`` rows,
     fold-ordered with ``fold_counts`` rows per fold (None: no folds).  The bands cover [0, n_rows), are cut at
     ``tile``-row boundaries and hold equal numbers of ADMISSIBLE tiles, counted as the tensor-core filter counts them
     with ``tile``-row query and database tiles: database tile b is computed for query tile a iff b >= a (triangle) and
     not both tiles lie inside the same fold.  A band of early rows is short, one of late rows long.  Ranks past the
-    number of tiles get empty bands."""
+    number of tiles get empty bands.
+    ``q_begin`` (a multiple of ``tile``) and ``q_end`` cut the sub-range [q_begin, q_end) into ``world`` such bands
+    instead: the sub-bands of one query band whose pairs overflow (``Engine.duplicate_groups``)."""
+    q_end = n_rows if q_end is None else int(q_end)
+    if q_begin % tile or not 0 <= q_begin <= q_end <= n_rows:
+        raise ValueError(f"self_join_ranges: need a {tile}-aligned 0 <= q_begin <= q_end <= n_rows, "
+                         f"got {q_begin}, {q_end}, {n_rows}")
     n_t = (n_rows + tile - 1) // tile
-    if n_t == 0:
-        return [(0, 0)] * world
+    t0, t1 = q_begin // tile, (q_end + tile - 1) // tile
+    if t1 == t0:
+        return [(q_begin, q_end)] * world
     a = np.arange(n_t, dtype=np.int64)
     cost = (n_t - a).astype(np.float64)                       # database tiles b >= a
     if fold_counts is not None:
@@ -278,10 +286,11 @@ def self_join_ranges(n_rows: int, fold_counts: Optional[Sequence[int]], world: i
         for f in np.unique(f_lo[single]):
             idx = np.nonzero(single & (f_lo == f))[0]
             cost[idx] -= len(idx) - np.arange(len(idx))
-    cum = np.concatenate([[0.0], np.cumsum(cost)])
-    cuts = [0] + [int(np.searchsorted(cum, cum[-1] * r / world, side="left")) for r in range(1, world)] + [n_t]
-    cuts = np.maximum.accumulate(np.minimum(cuts, n_t))
-    return [(min(int(cuts[r]) * tile, n_rows), min(int(cuts[r + 1]) * tile, n_rows)) for r in range(world)]
+    cum = np.concatenate([[0.0], np.cumsum(cost[t0:t1])])
+    n_sub = t1 - t0
+    cuts = [0] + [int(np.searchsorted(cum, cum[-1] * r / world, side="left")) for r in range(1, world)] + [n_sub]
+    cuts = np.maximum.accumulate(np.minimum(cuts, n_sub)) + t0
+    return [(min(int(cuts[r]) * tile, q_end), min(int(cuts[r + 1]) * tile, q_end)) for r in range(world)]
 
 
 def ranges_to_rows(ranges: Sequence[Tuple[int, int]], device) -> torch.Tensor:

@@ -863,39 +863,13 @@ class Engine:
         (verified with checksums): each rank prepares the whole cohort, joins its band of query rows
         (``dist.self_join_ranges``, equal tensor-core work per rank) and the pair lists are all-gathered; every rank
         returns the same result, bit for bit equal to ``distributed=False``."""
-        if not np.isfinite(min_score):
-            raise ValueError(f"near_duplicates: min_score must be finite, got {min_score}")
-        mats = [self._embedding(x)[0] for x in segs if x is not None]
-        n = int(mats[0].shape[0])
-        folds_t, perm = None, None
-        if folds is not None:
-            folds_t = self.to_device(folds, torch.uint8)
-            if int(folds_t.shape[0]) != n:
-                raise ValueError(f"near_duplicates: {int(folds_t.shape[0])} fold ids for {n} rows")
-            perm = _fold_order(folds_t)
-            if perm is not None:
-                mats = [m.index_select(0, perm) for m in mats]
-                folds_t = folds_t.index_select(0, perm)
+        mats, n, folds_t, perm = self._self_join_rows(segs, min_score, folds, "near_duplicates")
         q0, q1, world = 0, n, 1
         if distributed:
             import torch.distributed as tdist
             from .dist import self_join_ranges
             world, rank = tdist.get_world_size(), tdist.get_rank()
-            # cheap guard against ranks that were handed different cohorts
-            sample = torch.arange(0, n, max(1, n // 61), device=self.device)[:64]
-            sig = torch.stack([torch.tensor(float(n), device=self.device, dtype=torch.float64),
-                               torch.tensor(float(sum(int(m.shape[1]) for m in mats)), device=self.device,
-                                            dtype=torch.float64),
-                               folds_t.double().sum() if folds_t is not None else torch.zeros((), device=self.device,
-                                                                                              dtype=torch.float64)]
-                              + [m.index_select(0, sample).double().sum() for m in mats])
-            lo_sig, hi_sig = sig.clone(), sig.clone()
-            tdist.all_reduce(lo_sig, op=tdist.ReduceOp.MIN)
-            tdist.all_reduce(hi_sig, op=tdist.ReduceOp.MAX)
-            if not torch.equal(lo_sig, hi_sig):
-                raise ValueError("near_duplicates(distributed=True): the ranks were called with different cohorts "
-                                 "(row count / dim / fold / row-sample checksums differ); every rank must pass the same "
-                                 "arrays")
+            self._check_same_cohort(mats, folds_t, n, "near_duplicates")
             counts = None if folds_t is None else torch.bincount(folds_t.long()).cpu().tolist()
             q0, q1 = self_join_ranges(n, counts, world)[rank]
         op = self.prepare(mats[0], mats[1] if len(mats) > 1 else None, 1.0, 1.0, flags, "rescore")
@@ -906,16 +880,60 @@ class Engine:
             err, pairs = None, torch.zeros((0, 2), dtype=torch.int64, device=self.device)
             try:
                 pairs = self.self_join_prepared(op, min_score, folds_t, q0, q1, max_results)
-            except ValueError as e:             # every rank must take the same branch: the collectives below must match
+            except ValueError as e:
                 err = e
-            failed = torch.tensor([0 if err is None else 1], dtype=torch.int64, device=self.device)
-            tdist.all_reduce(failed, op=tdist.ReduceOp.MAX)
-            if int(failed.item()):
-                raise err if err is not None else ValueError("near_duplicates: another rank's band exceeded max_results")
+            self._raise_on_every_rank(err, "near_duplicates: another rank's band exceeded max_results")
             pairs = torch.cat(_gather_varlen(pairs, world))
             if int(pairs.shape[0]) > max_results:
                 raise ValueError(f"near_duplicates: {int(pairs.shape[0])} pairs exceed max_results = {max_results}")
         return self_join_result(pairs, perm, folds_t, n)
+
+    def _self_join_rows(self, segs: Sequence, min_score: float, folds, who: str
+                        ) -> Tuple[List[torch.Tensor], int, Optional[torch.Tensor], Optional[torch.Tensor]]:
+        """The rows of a self-join as device matrices (one per modality), brought into fold order when ``folds`` is
+        given: (matrices, n, folds in that order or None, perm or None; ``perm[r]`` = caller row of joined row r)."""
+        if not np.isfinite(min_score):
+            raise ValueError(f"{who}: min_score must be finite, got {min_score}")
+        mats = [self._embedding(x)[0] for x in segs if x is not None]
+        n = int(mats[0].shape[0])
+        folds_t, perm = None, None
+        if folds is not None:
+            folds_t = self.to_device(folds, torch.uint8)
+            if int(folds_t.shape[0]) != n:
+                raise ValueError(f"{who}: {int(folds_t.shape[0])} fold ids for {n} rows")
+            perm = _fold_order(folds_t)
+            if perm is not None:
+                mats = [m.index_select(0, perm) for m in mats]
+                folds_t = folds_t.index_select(0, perm)
+        return mats, n, folds_t, perm
+
+    def _check_same_cohort(self, mats: Sequence[torch.Tensor], folds_t: Optional[torch.Tensor], n: int, who: str) -> None:
+        """Cheap guard of a distributed self-join against ranks that were handed different cohorts: row count, dim,
+        fold sum and a row sample are compared over the ranks (all-reduce MIN and MAX)."""
+        import torch.distributed as tdist
+        sample = torch.arange(0, n, max(1, n // 61), device=self.device)[:64]
+        sig = torch.stack([torch.tensor(float(n), device=self.device, dtype=torch.float64),
+                           torch.tensor(float(sum(int(m.shape[1]) for m in mats)), device=self.device,
+                                        dtype=torch.float64),
+                           folds_t.double().sum() if folds_t is not None else torch.zeros((), device=self.device,
+                                                                                          dtype=torch.float64)]
+                          + [m.index_select(0, sample).double().sum() for m in mats])
+        lo_sig, hi_sig = sig.clone(), sig.clone()
+        tdist.all_reduce(lo_sig, op=tdist.ReduceOp.MIN)
+        tdist.all_reduce(hi_sig, op=tdist.ReduceOp.MAX)
+        if not torch.equal(lo_sig, hi_sig):
+            raise ValueError(f"{who}(distributed=True): the ranks were called with different cohorts "
+                             "(row count / dim / fold / row-sample checksums differ); every rank must pass the same "
+                             "arrays")
+
+    def _raise_on_every_rank(self, err: Optional[Exception], other_text: str) -> None:
+        """Every rank must take the same branch, or the collectives that follow would not match: a rank's error is
+        all-reduced, and every rank raises (its own error, or ``other_text`` when another rank failed)."""
+        import torch.distributed as tdist
+        failed = torch.tensor([0 if err is None else 1], dtype=torch.int64, device=self.device)
+        tdist.all_reduce(failed, op=tdist.ReduceOp.MAX)
+        if int(failed.item()):
+            raise err if err is not None else ValueError(other_text)
 
     def self_join_prepared(self, op: Operand, min_score: float, folds=None, q_begin: int = 0, q_end: Optional[int] = None,
                            max_results: int = 1 << 26) -> torch.Tensor:
@@ -945,6 +963,170 @@ class Engine:
                 int(fold_sorted), float(min_score), op.stats.data_ptr(), cand.data_ptr(), cand_cap, out.data_ptr(),
                 res_cap, counts.data_ptr(), _round_up(ws.data_ptr(), 256), ws_bytes, self._stream())
         return self._pairs_with_retry(call, min(max_results, max(1 << 16, q_end - q_begin)), max_results, "self_join")
+
+    # ------------------------------------------------- near-duplicate groups
+    def _components_union(self, parent: torch.Tensor, edges: torch.Tensor, bad: torch.Tensor) -> None:
+        """``emr2a_components_union``: fold the int64 edges [m, 2] into the forest ``parent`` (in place); edges with an
+        end outside [0, n) are counted in ``bad`` (int64 [1], zeroed by the caller)."""
+        with torch.cuda.device(self.device):
+            native.check(self.lib.emr2a_components_union(parent.data_ptr(), int(parent.shape[0]), edges.data_ptr(),
+                                                         int(edges.shape[0]), bad.data_ptr(), self._stream()))
+        self.launches += 1 if int(edges.shape[0]) else 0
+
+    def _components_finish(self, parent: torch.Tensor) -> None:
+        """``emr2a_components_finish``: parent[v] = the smallest vertex of v's component, in place."""
+        with torch.cuda.device(self.device):
+            native.check(self.lib.emr2a_components_finish(parent.data_ptr(), int(parent.shape[0]), self._stream()))
+        self.launches += 1 if int(parent.shape[0]) else 0
+
+    def connected_components(self, edges, n: int, parent: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Connected components of the undirected graph on vertices [0, n) with ``edges`` (int64 [m, 2], pairs (a, b))
+        on the GPU.  Returns int64 [n]: the label of v is the smallest vertex of v's component, whatever the edge
+        order.  ``parent`` (int64 [n] on this device, 0 <= parent[v] <= v) starts from an earlier result instead of
+        arange(n) -- the components of the union of both edge sets -- and is updated in place.  Raises ValueError if an edge has an
+        end outside [0, n) (nothing is changed for such an edge)."""
+        n = int(n)
+        if n < 0:
+            raise ValueError(f"connected_components: n must be >= 0, got {n}")
+        edges = self.to_device(edges, torch.int64)
+        if edges.numel() == 0:
+            edges = edges.reshape(0, 2)
+        if edges.dim() != 2 or int(edges.shape[1]) != 2:
+            raise ValueError(f"connected_components: edges must have shape [m, 2], got {tuple(edges.shape)}")
+        if parent is None:
+            parent = torch.arange(n, dtype=torch.int64, device=self.device)
+        elif parent.dtype != torch.int64 or parent.device != self.device or tuple(parent.shape) != (n,) \
+                or not parent.is_contiguous():
+            raise ValueError(f"connected_components: parent must be a contiguous int64 [{n}] tensor on {self.device}")
+        elif n and not bool(((parent >= 0) & (parent <= torch.arange(n, device=self.device))).all()):
+            raise ValueError("connected_components: parent must be a forest with 0 <= parent[v] <= v")
+        bad = torch.zeros((1,), dtype=torch.int64, device=self.device)
+        self._components_union(parent, edges, bad)
+        self._components_finish(parent)
+        n_bad = int(bad.item())
+        if n_bad:
+            raise ValueError(f"connected_components: {n_bad} edges have an end outside [0, {n})")
+        return parent
+
+    def _union_band(self, op: Operand, min_score: float, parent: torch.Tensor, bad: torch.Tensor, q0: int, q1: int,
+                    pair_budget: int) -> Dict[str, int]:
+        """Self-join the query band [q0, q1) and fold its pairs into ``parent``, one sub-band at a time so that no
+        sub-band holds more than ``pair_budget`` pairs (or 4 x as many filter candidates).  The first pass takes the
+        whole band; a band that overflows with c pairs is cut into ceil(2 c / pair_budget) 256-aligned sub-bands of
+        equal admissible tiles (``dist.self_join_ranges``; at most one per 256-row tile of the band), which are run in
+        turn and cut again if they overflow.
+        Returns the counts: ``pairs`` (s >= t), ``bands`` (passes that completed), ``overflows`` (passes that did
+        not)."""
+        from .dist import self_join_ranges
+        todo, out = [(q0, q1)], {"pairs": 0, "bands": 0, "overflows": 0}
+        while todo:
+            b0, b1 = todo.pop(0)
+            try:
+                pairs = self.self_join_prepared(op, min_score, None, b0, b1, pair_budget)
+            except PairOverflow as e:
+                out["overflows"] += 1
+                # more parts than the band has 256-row tiles would only be empty ones
+                parts = min(-(-2 * e.pairs // pair_budget), -(-(b1 - b0) // 256))
+                sub = [r for r in self_join_ranges(op.n, None, parts, q_begin=b0, q_end=b1) if r[1] > r[0]]
+                if len(sub) < 2:
+                    raise ValueError(f"duplicate_groups: the query band [{b0}, {b1}) cannot be split further and has "
+                                     f"{e.pairs} pairs, more than pair_budget = {pair_budget}; raise min_score or "
+                                     "pair_budget") from e
+                todo = sub + todo
+                continue
+            out["bands"] += 1
+            out["pairs"] += int(pairs.shape[0])
+            if pairs.shape[0]:
+                _, j = decode_keys(pairs[:, 1])
+                self._components_union(parent, torch.stack([pairs[:, 0], j], dim=1), bad)
+            del pairs
+        return out
+
+    def duplicate_groups(self, segs: Sequence, min_score: float, flags: int = native.NF_ROWNORM,
+                         pair_budget: int = 1 << 26, distributed: bool = False) -> Dict[str, object]:
+        """Groups of near-duplicate rows: the connected components of the graph whose edges are the pairs
+        ``near_duplicates`` returns (exact fp32 similarity >= ``min_score``, rows prepared the same way).  a ~ b and
+        b ~ c put a, b and c in one group even when a and c score below ``min_score`` (single linkage).
+        The self-join runs in query bands whose pairs are folded into a union-find on the GPU
+        (``connected_components``) and dropped, so the pair list is never held: a band with more than ``pair_budget``
+        pairs is cut into smaller bands and run again, and only a single 256-row band above the budget raises
+        ValueError.
+        Returns ``group`` int64 [n] (the smallest row of the row's group; ``group[i] == i`` for a row without
+        partners), ``keep`` bool [n] (one row per group: ``group == arange(n)``), ``group_size`` int64 [n],
+        ``n_groups`` and ``n_pairs`` (pairs with s >= t), and ``n_bands`` / ``n_overflows`` (self-join passes that
+        completed / that overflowed and were split).  The labels do not depend on the band plan or the GPU count.
+        ``distributed=True``: under ``torchrun`` with an NCCL process group, every rank called with the same arrays
+        (checked as in ``near_duplicates``): each rank joins its band (``dist.self_join_ranges``) into a forest of its
+        own, the non-trivial labels are all-gathered and every rank merges them; every rank returns the same result,
+        bit for bit equal to ``distributed=False``."""
+        mats, n, _, _ = self._self_join_rows(segs, min_score, None, "duplicate_groups")
+        return self._groups_of_rows(mats, n, None, min_score, flags, pair_budget, distributed, "duplicate_groups")
+
+    def _groups_of_rows(self, mats: Sequence[torch.Tensor], n: int, folds_t: Optional[torch.Tensor], min_score: float,
+                        flags: int, pair_budget: int, distributed: bool, who: str) -> Dict[str, object]:
+        """``duplicate_groups`` on the device matrices of ``_self_join_rows``.  ``folds_t`` (caller row order) only
+        joins the distributed cohort guard; the groups never depend on it."""
+        pair_budget = int(pair_budget)
+        if pair_budget < 1:
+            raise ValueError(f"{who}: pair_budget must be >= 1, got {pair_budget}")
+        q0, q1, world = 0, n, 1
+        if distributed:
+            import torch.distributed as tdist
+            from .dist import self_join_ranges
+            world, rank = tdist.get_world_size(), tdist.get_rank()
+            self._check_same_cohort(mats, folds_t, n, who)
+            q0, q1 = self_join_ranges(n, None, world)[rank]
+        op = self.prepare(mats[0], mats[1] if len(mats) > 1 else None, 1.0, 1.0, flags, "rescore")
+        parent = torch.arange(n, dtype=torch.int64, device=self.device)
+        bad = torch.zeros((1,), dtype=torch.int64, device=self.device)
+        if world == 1:
+            counts = self._union_band(op, min_score, parent, bad, q0, q1, pair_budget)
+        else:
+            from .dist import _gather_varlen
+            err, counts = None, {"pairs": 0, "bands": 0, "overflows": 0}
+            try:
+                counts = self._union_band(op, min_score, parent, bad, q0, q1, pair_budget)
+            except ValueError as e:
+                err = e
+            self._raise_on_every_rank(err, f"{who}: another rank's band could not be split below pair_budget")
+            self._components_finish(parent)
+            # the components of the union of the per-rank forests are the global components
+            v = torch.nonzero(parent != torch.arange(n, dtype=torch.int64, device=self.device)).squeeze(1)
+            links = torch.cat(_gather_varlen(torch.stack([v, parent[v]], dim=1), world))
+            parent = torch.arange(n, dtype=torch.int64, device=self.device)
+            self._components_union(parent, links, bad)
+            tot = torch.tensor([counts["pairs"], counts["bands"], counts["overflows"]], dtype=torch.int64,
+                               device=self.device)
+            tdist.all_reduce(tot)
+            counts = dict(zip(("pairs", "bands", "overflows"), (int(x) for x in tot.cpu().tolist())))
+        self._components_finish(parent)
+        if int(bad.item()):
+            raise RuntimeError(f"duplicate_groups: {int(bad.item())} self-join pairs decoded outside [0, {n})")
+        keep = parent == torch.arange(n, dtype=torch.int64, device=self.device)
+        size = torch.bincount(parent, minlength=n)[parent] if n else torch.zeros(0, dtype=torch.int64,
+                                                                                  device=self.device)
+        return {"group": parent, "keep": keep, "group_size": size, "n_groups": int(keep.sum().item()),
+                "n_pairs": counts["pairs"], "n_bands": counts["bands"], "n_overflows": counts["overflows"]}
+
+    def leak_free_folds(self, segs: Sequence, folds, min_score: float, flags: int = native.NF_ROWNORM,
+                        pair_budget: int = 1 << 26, distributed: bool = False) -> Dict[str, torch.Tensor]:
+        """A CV fold assignment without near-duplicate leaks: every group of ``duplicate_groups`` moves into the fold
+        of its smallest row, ``new[i] = folds[group[i]]``.  Rows without partners keep the caller's fold.
+        Guarantee: ``cross_fold_duplicates(segs, new_folds, min_score)`` with the same flags returns no pairs.  Every
+        pair with s >= min_score is an edge of the graph, so its ends share a group and therefore a fold; the
+        self-join's exact scores do not depend on the row order, so this holds exactly.
+        Fold sizes are not rebalanced.  Returns ``folds`` uint8 [n], ``moved`` int64 (rows whose fold changed),
+        ``group`` int64 [n], and ``fold_counts_before`` / ``fold_counts_after`` (int64, one per fold)."""
+        mats, n, _, _ = self._self_join_rows(segs, min_score, None, "leak_free_folds")
+        folds_t = self.to_device(folds, torch.uint8)
+        if int(folds_t.shape[0]) != n:
+            raise ValueError(f"leak_free_folds: {int(folds_t.shape[0])} fold ids for {n} rows")
+        g = self._groups_of_rows(mats, n, folds_t, min_score, flags, pair_budget, distributed, "leak_free_folds")
+        new = folds_t[g["group"]]
+        n_folds = int(folds_t.max().item()) + 1 if n else 0
+        return {"folds": new, "moved": torch.nonzero(new != folds_t).squeeze(1), "group": g["group"],
+                "fold_counts_before": torch.bincount(folds_t.long(), minlength=n_folds),
+                "fold_counts_after": torch.bincount(new.long(), minlength=n_folds)}
 
     # ----------------------------------------------- host-buffer (end-to-end) path
     def search_and_vote_host(self, db_segs_host: Sequence, q_segs_host: Sequence, db_labels, q_labels,
@@ -1073,19 +1255,28 @@ def csr_from_pairs(pairs: torch.Tensor, n_queries: int) -> Dict[str, torch.Tenso
     return {"offsets": offsets, "idx": idx, "scores": scores}
 
 
+class PairOverflow(ValueError):
+    """A range search or self-join found more pairs than its caller allows.  ``pairs`` is the size of the overflow in
+    results: the exact result count, or a quarter of the candidate count when the filter candidates overflowed."""
+
+    def __init__(self, text: str, pairs: int):
+        super().__init__(text)
+        self.pairs = int(pairs)
+
+
 def range_retry_caps(n_cand: int, n_res: int, cand_cap: int, res_cap: int, max_results: int
                      ) -> Optional[Tuple[int, int]]:
     """Buffer sizes for the one retry of a range search (None: the outputs are complete).  The counts of
     emr2a_range_search are exact; when the candidates overflowed nothing was re-scored and the results, a subset of
-    the candidates, are bounded by their count.  Raises ValueError instead of sizing past ``max_results`` results or
-    4 x ``max_results`` candidates."""
+    the candidates, are bounded by their count.  Raises PairOverflow (a ValueError) instead of sizing past
+    ``max_results`` results or 4 x ``max_results`` candidates."""
     if n_cand > 4 * max_results:
-        raise ValueError(f"range_search: {n_cand} filter candidates exceed 4 x max_results = {4 * max_results}; "
-                         "raise min_score or max_results")
+        raise PairOverflow(f"range_search: {n_cand} filter candidates exceed 4 x max_results = {4 * max_results}; "
+                           "raise min_score or max_results", (n_cand + 3) // 4)
     if n_cand > cand_cap:
         return n_cand, max(1, min(n_cand, max_results))
     if n_res > max_results:
-        raise ValueError(f"range_search: {n_res} results exceed max_results = {max_results}")
+        raise PairOverflow(f"range_search: {n_res} results exceed max_results = {max_results}", n_res)
     if n_res > res_cap:
         return cand_cap, n_res
     return None

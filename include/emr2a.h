@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define EMR2A_ABI_VERSION 13
+#define EMR2A_ABI_VERSION 14
 
 enum emr2a_status {
   EMR2A_OK = 0,
@@ -323,6 +323,24 @@ int emr2a_self_join(const float* x_f32, int64_t ld_f32, const uint16_t* x_hi, in
                     int64_t q_begin, int64_t q_end, const uint8_t* fold, int fold_sorted, float min_score,
                     const float* stats, uint64_t* cand, int64_t cand_cap, uint64_t* results, int64_t result_cap,
                     uint64_t* counts_out, void* workspace, size_t ws_bytes, void* stream);
+
+/*
+ * Connected components of an undirected edge list: a union-find over a caller-owned parent [n] (int64, device).
+ * parent may hold any forest with parent[v] <= v: arange(n) to start, or the output of an earlier finish.
+ *   emr2a_components_union   folds the edges [m][2] (a, b) into the forest.  It may be called any number of times on
+ *                            the same state before the finish (the near-duplicate groups fold in one query band of the
+ *                            self-join at a time).  Self-loops and duplicate edges are harmless.  An edge with an end
+ *                            outside [0, n) is skipped and counted in bad_edges_out [1] (uint64, zeroed by the caller).
+ *   emr2a_components_finish  sets parent[v] to the root of v, in place.
+ * After the finish parent[v] is the SMALLEST vertex of v's component: a canonical label that does not depend on the
+ * order of the edges, on how they were split over calls, or on the thread schedule.
+ * Both calls are stream-ordered; they neither synchronise nor allocate.
+ * Errors (before anything is launched): EMR2A_ERR_INVALID for n < 0, m < 0, a NULL pointer where its size is > 0
+ * (bad_edges_out counts when m > 0), or n >= 2^32 - 1 (the row limit of the packed keys).
+ */
+int emr2a_components_union(int64_t* parent, int64_t n, const int64_t* edges, int64_t m, uint64_t* bad_edges_out,
+                           void* stream);
+int emr2a_components_finish(int64_t* parent, int64_t n, void* stream);
 
 /*
  * K3 -- merge `parts` partial Top-K lists per query into one.  Every input list must be sorted

@@ -107,5 +107,23 @@ for name, f in (("no folds", None), ("unsorted folds", sj_folds)):
     print(f"rank {rank}/{world} near_duplicates {name}: distributed == single-GPU: {same} ({int(b['i'].numel())} pairs)",
           flush=True)
     ok = ok and same and int(b["i"].numel()) > 0
+# near-duplicate groups: each rank folds its band into a forest of its own, the forests are merged on every rank;
+# a chain through both halves of the cohort joins rows of different ranks' bands, a tiny budget splits the bands
+xs[n_sj - 700:n_sj - 200] = xs[n_sj // 2:n_sj // 2 + 500] + 1e-3 * xs[1000:1500]
+for budget in (1 << 26, 600):
+    a = eng.duplicate_groups([xs], 0.999, pair_budget=budget, distributed=True)
+    b = eng.duplicate_groups([xs], 0.999, distributed=False)
+    same = all(torch.equal(a[key], b[key]) for key in ("group", "keep", "group_size")) and \
+        (a["n_groups"], a["n_pairs"]) == (b["n_groups"], b["n_pairs"])
+    print(f"rank {rank}/{world} duplicate_groups pair_budget={budget}: distributed == single-GPU: {same} "
+          f"({b['n_groups']} groups, {b['n_pairs']} pairs, {a['n_bands']} bands)", flush=True)
+    ok = ok and same and b["n_groups"] < n_sj
+a = eng.leak_free_folds([xs], sj_folds, 0.999, distributed=True)
+b = eng.leak_free_folds([xs], sj_folds, 0.999, distributed=False)
+same = all(torch.equal(a[key], b[key]) for key in b)
+clean = int(eng.cross_fold_duplicates([xs], a["folds"], 0.999)["i"].numel()) == 0
+print(f"rank {rank}/{world} leak_free_folds: distributed == single-GPU: {same}, no cross-fold pair left: {clean} "
+      f"({int(a['moved'].numel())} rows moved)", flush=True)
+ok = ok and same and clean
 dist.barrier(); dist.destroy_process_group()
 sys.exit(0 if ok else 1)
