@@ -90,6 +90,13 @@ __global__ void zero_keys_kernel(uint64_t* k, int64_t n) {
   if (i < n) k[i] = 0ull;
 }
 
+// the key lists of an empty database: n empty keys
+static int zero_keys(uint64_t* k, int64_t n, cudaStream_t st) {
+  zero_keys_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(k, n);
+  EMR2A_LAUNCH_CHECK("zero_keys_kernel");
+  return EMR2A_OK;
+}
+
 }  // namespace emr2a
 
 using namespace emr2a;
@@ -171,12 +178,7 @@ static int topk_search_impl(const float* q_f32, int64_t ldq_f32, const uint16_t*
   if (idx_base < 0) return fail(EMR2A_ERR_INVALID, "topk_search: negative idx_base");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (Q == 0) return EMR2A_OK;
-  if (N == 0) {
-    const int64_t n = Q * K;
-    zero_keys_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(out_keys, n);
-    EMR2A_LAUNCH_CHECK("zero_keys_kernel");
-    return EMR2A_OK;
-  }
+  if (N == 0) return zero_keys(out_keys, Q * K, st);
   switch (precision) {
     case EMR2A_PREC_FP32:
       if (!q_f32 || !db_f32) return fail(EMR2A_ERR_INVALID, "topk_search(fp32): q_f32/db_f32 required");
@@ -261,9 +263,8 @@ extern "C" int emr2a_topk_filter(const uint16_t* q_hi, int64_t ldq_bf16, const u
   if (Q == 0) return EMR2A_OK;
   EMR2A_CUDA_TRY(cudaMemsetAsync(tau_out, 0, sizeof(uint32_t) * static_cast<size_t>(Q), st));
   if (N == 0) {
-    const int64_t n = Q * RESCORE_KPM;
-    zero_keys_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(cand_out, n);
-    EMR2A_LAUNCH_CHECK("zero_keys_kernel");
+    const int rc = zero_keys(cand_out, Q * RESCORE_KPM, st);
+    if (rc != EMR2A_OK) return rc;
   } else {
     if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) return fail(EMR2A_ERR_INVALID, "topk_filter: workspace must be 256-byte aligned");
     const uint64_t* cand = nullptr;
@@ -317,14 +318,21 @@ extern "C" int emr2a_exact_rescan(const float* q_f32, int64_t ldq_f32, const flo
   if ((q_fold == nullptr) != (db_fold == nullptr)) return fail(EMR2A_ERR_INVALID, "exact_rescan: q_fold and db_fold must be given together");
   if (n_flagged == 0) return EMR2A_OK;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (N == 0) {
-    const int64_t n = static_cast<int64_t>(n_flagged) * K;
-    zero_keys_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(out_keys, n);
-    EMR2A_LAUNCH_CHECK("zero_keys_kernel");
-    return EMR2A_OK;
-  }
+  if (N == 0) return zero_keys(out_keys, static_cast<int64_t>(n_flagged) * K, st);
   return rescore_exact_rescan(q_f32, ldq_f32, db_f32, lddb_f32, db_lazy, N, D, idx_base, K, q_fold, db_fold, flag_list,
                               n_flagged, out_keys, workspace, ws_bytes, db_hi, lddb_bf16, q_stats, db_stats, seed_keys, st);
+}
+
+// The tensor-core filter of a range search or self-join, then range_refine of its candidates.  The kernel timing ring
+// gets two entries: the filter (tc_range_filter records it around its launch) and the refine kernel.
+template <class Filter, class Refine>
+static int filter_then_refine(Filter filter, Refine refine, cudaStream_t st) {
+  int rc = filter();
+  if (rc != EMR2A_OK) return rc;
+  tc_timing_record(0, st);
+  rc = refine();
+  tc_timing_record(1, st);
+  return rc;
 }
 
 // ---- range search: every admissible pair with exact score >= min_score --------------------------------------------
@@ -356,14 +364,12 @@ extern "C" int emr2a_range_search(const float* q_f32, int64_t ldq_f32, const uin
   if (rc != EMR2A_OK) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   unsigned long long* counts = reinterpret_cast<unsigned long long*>(counts_out);
-  rc = tc_range_filter(q_hi, db_hi, Q, N, D, ldq_bf16, lddb_bf16, q_fold, db_fold, fold_sorted, idx_base, min_score,
-                           q_stats, db_stats, cand, cand_cap, counts, workspace, ws_bytes, st, false, 0);
-  if (rc != EMR2A_OK) return rc;
-  tc_timing_record(0, st);
-  rc = range_refine(cand, cand_cap, counts, results, result_cap, q_f32, ldq_f32, db_f32, lddb_f32, db_lazy, D, idx_base,
-                    min_score, st);
-  tc_timing_record(1, st);
-  return rc;
+  return filter_then_refine(
+      [&] { return tc_range_filter(q_hi, db_hi, Q, N, D, ldq_bf16, lddb_bf16, q_fold, db_fold, fold_sorted, idx_base,
+                                   min_score, q_stats, db_stats, cand, cand_cap, counts, workspace, ws_bytes, st, false, 0); },
+      [&] { return range_refine(cand, cand_cap, counts, results, result_cap, q_f32, ldq_f32, db_f32, lddb_f32, db_lazy, D,
+                                idx_base, min_score, st); },
+      st);
 }
 
 // ---- self-join: every pair i < j of one row set with exact score >= min_score ----------------------------------------
@@ -393,14 +399,14 @@ extern "C" int emr2a_self_join(const float* x_f32, int64_t ld_f32, const uint16_
   // queries [q_begin, q_end) against rows [q_begin, n): no row below q_begin is a partner j > i of these queries
   const uint16_t* band = x_hi + q_begin * ld_bf16;
   const uint8_t* band_fold = fold ? fold + q_begin : nullptr;
-  rc = tc_range_filter(band, band, q_end - q_begin, n - q_begin, D, ld_bf16, ld_bf16, band_fold, band_fold, fold_sorted,
-                       q_begin, min_score, stats, stats, cand, cand_cap, counts, workspace, ws_bytes, st, true, q_begin);
-  if (rc != EMR2A_OK) return rc;
-  tc_timing_record(0, st);
   // candidates carry global rows on both sides: re-scored against the whole row set
-  rc = range_refine(cand, cand_cap, counts, results, result_cap, x_f32, ld_f32, x_f32, ld_f32, nullptr, D, 0, min_score, st);
-  tc_timing_record(1, st);
-  return rc;
+  return filter_then_refine(
+      [&] { return tc_range_filter(band, band, q_end - q_begin, n - q_begin, D, ld_bf16, ld_bf16, band_fold, band_fold,
+                                   fold_sorted, q_begin, min_score, stats, stats, cand, cand_cap, counts, workspace,
+                                   ws_bytes, st, true, q_begin); },
+      [&] { return range_refine(cand, cand_cap, counts, results, result_cap, x_f32, ld_f32, x_f32, ld_f32, nullptr, D, 0,
+                                min_score, st); },
+      st);
 }
 
 // Diagnostics: time the Top-K kernel of every search alone (CUDA events on the launching stream around its launch).

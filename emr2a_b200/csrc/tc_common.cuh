@@ -1,4 +1,5 @@
-// Device helpers shared by the single-CTA (topk_tc.cu) and CTA-pair (topk_tc2.cu) tcgen05 kernels.
+// Device helpers shared by the single-CTA (topk_tc.cu) and CTA-pair (topk_tc2.cu) tcgen05 kernels, and the list of
+// their instantiations that both launch paths dispatch over.
 #pragma once
 #include <cuda.h>
 #include "common.cuh"
@@ -371,6 +372,23 @@ __device__ __forceinline__ float unit_start_threshold(const TcParams& p, int64_t
   if (b > 0.f) return __uint_as_float(bits - 1u);
   if (b < 0.f) return __uint_as_float(bits + 1u);
   return -1e-45f;                                 // just below zero
+}
+
+// ---- host: the instantiations of both kernels ------------------------------------------------------------------------
+// Every instantiation of tc_topk_kernel and tc2_topk_kernel has this type.
+typedef void (*TcKernel)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, TcParams);
+
+// The instantiations that exist, the same for both kernels: Top-K with passes {1, 3} x register list {8, 16, 32}, and
+// the range epilogue with 1 pass (its register list is unused: KCAP 8); each with and without folds.
+// K<PASSES, KCAP, RANGE>::get(fold) names one of them.  Any other combination gets null.
+template <template <int, int, bool> class K>
+static TcKernel tc_pick(int passes, int kcap, bool fold, bool range) {
+  if (range) return passes == 1 && kcap == 8 ? K<1, 8, true>::get(fold) : nullptr;
+  if (passes == 1)
+    return kcap == 8 ? K<1, 8, false>::get(fold) : kcap == 16 ? K<1, 16, false>::get(fold) : kcap == 32 ? K<1, 32, false>::get(fold) : nullptr;
+  if (passes == 3)
+    return kcap == 8 ? K<3, 8, false>::get(fold) : kcap == 16 ? K<3, 16, false>::get(fold) : kcap == 32 ? K<3, 32, false>::get(fold) : nullptr;
+  return nullptr;
 }
 
 }  // namespace emr2a

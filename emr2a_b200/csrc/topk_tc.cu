@@ -248,8 +248,7 @@ __device__ unsigned long long g_unit_clock[2 * UNIT_CLOCK_MAX];
 static int64_t g_last_plan[8];
 
 // CTA-pair kernel (topk_tc2.cu)
-int tc2_dispatch(int passes, int kcap, bool has_fold, const CUtensorMap& a, const CUtensorMap& b, const CUtensorMap& c,
-                 const CUtensorMap& d, const TcParams& p, int grid, cudaStream_t st);
+TcKernel tc2_kernel(int passes, int kcap, bool fold, bool range, size_t* smem);
 
 // CTA pairs (M = 256 per tile, cta_group::2) or single CTAs (M = 128).  Pairs win whenever the tensor pipe is the
 // bound (one third less L2->SM traffic per FLOP).  A batch of up to 128 queries is HBM-bound -- the database plane is
@@ -400,26 +399,6 @@ int tc_timing_read(float* ms_out, int cap, int* n_out) {
   return EMR2A_OK;
 }
 
-template <int PASSES, int KCAP, bool HAS_FOLD, bool RANGE = false>
-static int tc_launch(const CUtensorMap& mq_hi, const CUtensorMap& mq_lo, const CUtensorMap& md_hi, const CUtensorMap& md_lo,
-                     const TcParams& p, int grid, cudaStream_t st) {
-  constexpr int PLANES = PASSES == 3 ? 2 : 1;
-  constexpr int STAGES = PASSES == 3 ? 2 : 4;
-  const size_t smem = static_cast<size_t>(STAGES) * PLANES * (T_A_BYTES + T_B_BYTES) + 1024;
-  auto kern = tc_topk_kernel<PASSES, KCAP, HAS_FOLD, RANGE>;
-  EMR2A_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-  kern<<<grid, T_THREADS, smem, st>>>(mq_hi, mq_lo, md_hi, md_lo, p);
-  EMR2A_LAUNCH_CHECK("tc_topk_kernel");
-  return EMR2A_OK;
-}
-
-template <int PASSES, int KCAP>
-static int tc_launch_fold(bool has_fold, const CUtensorMap& a, const CUtensorMap& b, const CUtensorMap& c, const CUtensorMap& d,
-                          const TcParams& p, int grid, cudaStream_t st) {
-  return has_fold ? tc_launch<PASSES, KCAP, true>(a, b, c, d, p, grid, st)
-                  : tc_launch<PASSES, KCAP, false>(a, b, c, d, p, grid, st);
-}
-
 // Shape rules of the bf16 planes (K1 layout) shared by the Top-K and the range filter.
 static int check_planes(const char* who, const uint16_t* q_hi, const uint16_t* q_lo, const uint16_t* db_hi,
                         const uint16_t* db_lo, int64_t Q, int64_t N, int D, int64_t ldq, int64_t lddb, int64_t idx_base,
@@ -436,133 +415,59 @@ static int check_planes(const char* who, const uint16_t* q_hi, const uint16_t* q
   return EMR2A_OK;
 }
 
-int tc_topk_search(const uint16_t* q_hi, const uint16_t* q_lo, const uint16_t* db_hi, const uint16_t* db_lo,
-                   int64_t Q, int64_t N, int D, int64_t ldq, int64_t lddb,
-                   const uint8_t* q_fold, const uint8_t* db_fold, int64_t idx_base, int K, int passes,
-                   uint64_t* out_keys, void* workspace, size_t ws_bytes, float* debug_scores, cudaStream_t st,
-                   TcPartials* partials, int fold_sorted, int min_splits) {
-  if (K > 32) return fail(EMR2A_ERR_UNSUPPORTED, "topk_search(bf16): K=%d > 32 (use EMR2A_PREC_FP32)", K);
-  const int64_t Dp = (static_cast<int64_t>(D) + T_BK - 1) / T_BK * T_BK;
-  {
-    const int rc = check_planes("topk_search(bf16)", q_hi, q_lo, db_hi, db_lo, Q, N, D, ldq, lddb, idx_base, passes);
-    if (rc != EMR2A_OK) return rc;
-  }
-  const bool has_fold = q_fold != nullptr;
-  const bool pairs = use_cta_pairs(Q);
-  TcPlan pl = tc_plan(Q, N, K, has_fold, pairs, min_splits, lddb > ldq ? lddb : ldq, passes == 3 ? 2 : 1);
-  const size_t keys_off = 0;
-  const size_t fold_off = (pl.keys_bytes + 255) & ~static_cast<size_t>(255);
-  const size_t tau_off = (fold_off + pl.fold_bytes + 255) & ~static_cast<size_t>(255);
-  const size_t sync_off = tau_off + pl.tau_bytes;
-  const size_t need = sync_off + pl.sync_bytes;
-  if (!workspace || ws_bytes < need) return fail(EMR2A_ERR_WORKSPACE, "topk_search(bf16): workspace %zu < %zu", ws_bytes, need);
-  uint8_t* ws = static_cast<uint8_t*>(workspace);
-  if ((reinterpret_cast<uintptr_t>(ws) & 255) != 0) return fail(EMR2A_ERR_INVALID, "topk_search(bf16): workspace must be 256-byte aligned");
+// One launch of either kernel, as tc_setup prepared it.
+struct TcLaunch {
+  bool pairs;
+  TcPlan pl;
+  CUtensorMap mq_hi, mq_lo, md_hi, md_lo;       // 1 pass: the lo maps are copies of the hi maps
+  TcParams p;
+  uint64_t* keys;                                // the list-key region of the workspace (null without lists)
+};
 
-  CUtensorMap mq_hi, mq_lo, md_hi, md_lo;
-  int rc;
-  if ((rc = make_plane_map(&mq_hi, q_hi, Q, Dp, ldq, T_BM)) != EMR2A_OK) return rc;
+// Set-up shared by the Top-K search and the range filter: plane checks, plan, workspace, tensor maps, the common
+// TcParams fields, and the stream work before the kernel (tau and pacing memsets, fold padding).
+// Workspace, regions 256-byte aligned: list keys [splits][Q][K] | fold padding [n_tiles * 256] | tau [Q] | pacing
+// counters.  Without `lists` (range filter) the key and tau regions are empty.  Pacing runs whenever the workspace holds
+// its counters (it never changes a result); with `pacing_required` a workspace without them is an error.
+static int tc_setup(TcLaunch& L, const char* who, const uint16_t* q_hi, const uint16_t* q_lo, const uint16_t* db_hi,
+                    const uint16_t* db_lo, int64_t Q, int64_t N, int D, int64_t ldq, int64_t lddb, const uint8_t* q_fold,
+                    const uint8_t* db_fold, int fold_sorted, int64_t idx_base, int K, int passes, int min_splits, bool lists,
+                    bool pacing_required, void* workspace, size_t ws_bytes, cudaStream_t st) {
+  int rc = check_planes(who, q_hi, q_lo, db_hi, db_lo, Q, N, D, ldq, lddb, idx_base, passes);
+  if (rc != EMR2A_OK) return rc;
+  const int64_t Dp = (static_cast<int64_t>(D) + T_BK - 1) / T_BK * T_BK;
+  const bool has_fold = q_fold != nullptr;
+  const bool pairs = L.pairs = use_cta_pairs(Q);
+  L.pl = tc_plan(Q, N, K, has_fold, pairs, min_splits, lddb > ldq ? lddb : ldq, passes == 3 ? 2 : 1);
+  const TcPlan& pl = L.pl;
+  const size_t fold_off = ((lists ? pl.keys_bytes : 0) + 255) & ~static_cast<size_t>(255);
+  const size_t tau_off = (fold_off + pl.fold_bytes + 255) & ~static_cast<size_t>(255);
+  const size_t sync_off = tau_off + (lists ? pl.tau_bytes : 0);
+  const size_t need = sync_off + (pacing_required ? pl.sync_bytes : 0);
+  if (!workspace || ws_bytes < need) return fail(EMR2A_ERR_WORKSPACE, "%s: workspace %zu < %zu", who, ws_bytes, need);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  if ((reinterpret_cast<uintptr_t>(ws) & 255) != 0) return fail(EMR2A_ERR_INVALID, "%s: workspace must be 256-byte aligned", who);
+
+  if ((rc = make_plane_map(&L.mq_hi, q_hi, Q, Dp, ldq, T_BM)) != EMR2A_OK) return rc;
   const int db_box = pairs ? T_BN / 2 : T_BN;           // a CTA of a pair loads half of the database tile
-  if ((rc = make_plane_map(&md_hi, db_hi, N, Dp, lddb, db_box)) != EMR2A_OK) return rc;
+  if ((rc = make_plane_map(&L.md_hi, db_hi, N, Dp, lddb, db_box)) != EMR2A_OK) return rc;
   if (passes == 3) {
-    if ((rc = make_plane_map(&mq_lo, q_lo, Q, Dp, ldq, T_BM)) != EMR2A_OK) return rc;
-    if ((rc = make_plane_map(&md_lo, db_lo, N, Dp, lddb, db_box)) != EMR2A_OK) return rc;
+    if ((rc = make_plane_map(&L.mq_lo, q_lo, Q, Dp, ldq, T_BM)) != EMR2A_OK) return rc;
+    if ((rc = make_plane_map(&L.md_lo, db_lo, N, Dp, lddb, db_box)) != EMR2A_OK) return rc;
   } else {
-    mq_lo = mq_hi; md_lo = md_hi;
+    L.mq_lo = L.mq_hi; L.md_lo = L.md_hi;
   }
-  TcParams p{};
+  TcParams& p = L.p;
+  p = TcParams{};
   p.Q = Q; p.N = N; p.k_chunks = static_cast<int>(Dp / T_BK);
   p.m_tiles = pl.m_tiles; p.n_tiles = pl.n_tiles; p.splits = pl.splits; p.tiles_per_split = pl.tiles_per_split;
-  p.idx_base = idx_base; p.K = K; p.debug_scores = debug_scores;
-  p.keys_out = (pl.splits > 1 || partials) ? reinterpret_cast<uint64_t*>(ws + keys_off) : out_keys;
-  if (pl.splits > 1) {     // sharing only pays (and is only needed) when a query tile is searched by several units
+  p.idx_base = idx_base; p.K = K; p.mg = pl.mg;
+  L.keys = lists ? reinterpret_cast<uint64_t*>(ws) : nullptr;
+  if (lists && pl.splits > 1) {     // sharing only pays (and is only needed) when a query tile is searched by several units
     p.tau = reinterpret_cast<uint32_t*>(ws + tau_off);
     EMR2A_CUDA_TRY(cudaMemsetAsync(p.tau, 0, sizeof(uint32_t) * static_cast<size_t>(Q), st));
   }
-  p.mg = pl.mg;
-  if (pairs && pl.sync_bytes) {
-    p.sync_tiles = pl.sync_tiles; p.sync_points = pl.sync_points; p.sync_budget = pl.sync_budget;
-    p.sync_ctr = reinterpret_cast<uint32_t*>(ws + sync_off);
-    EMR2A_CUDA_TRY(cudaMemsetAsync(p.sync_ctr, 0, pl.sync_bytes, st));
-  }
-  if (pairs && env_int("EMR2A_TC_UNIT_CLOCK", 0) && pl.m_tiles * pl.splits <= UNIT_CLOCK_MAX) {
-    void* sym = nullptr;
-    EMR2A_CUDA_TRY(cudaGetSymbolAddress(&sym, g_unit_clock));
-    p.unit_clock = static_cast<unsigned long long*>(sym);
-    const int64_t plan[8] = {pl.m_tiles, pl.n_tiles, pl.splits, pl.tiles_per_split, pl.mg, pl.sync_tiles, pl.grid,
-                             pl.m_tiles * pl.splits};
-    for (int i = 0; i < 8; ++i) g_last_plan[i] = plan[i];
-  }
-  if (has_fold) {
-    uint8_t* fpad = ws + fold_off;
-    EMR2A_CUDA_TRY(cudaMemsetAsync(fpad, 0xFF, pl.fold_bytes, st));
-    EMR2A_CUDA_TRY(cudaMemcpyAsync(fpad, db_fold, static_cast<size_t>(N), cudaMemcpyDeviceToDevice, st));
-    p.q_fold = q_fold; p.db_fold = fpad; p.fold_sorted = fold_sorted;
-  }
-  const int kcap = K <= 8 ? 8 : (K <= 16 ? 16 : 32);
-  tc_ev_record(0, st);
-  if (pairs) {
-    rc = tc2_dispatch(passes, kcap, has_fold, mq_hi, mq_lo, md_hi, md_lo, p, pl.grid, st);
-  } else if (passes == 3) {
-    if (kcap == 8) rc = tc_launch_fold<3, 8>(has_fold, mq_hi, mq_lo, md_hi, md_lo, p, pl.grid, st);
-    else if (kcap == 16) rc = tc_launch_fold<3, 16>(has_fold, mq_hi, mq_lo, md_hi, md_lo, p, pl.grid, st);
-    else rc = tc_launch_fold<3, 32>(has_fold, mq_hi, mq_lo, md_hi, md_lo, p, pl.grid, st);
-  } else {
-    if (kcap == 8) rc = tc_launch_fold<1, 8>(has_fold, mq_hi, mq_lo, md_hi, md_lo, p, pl.grid, st);
-    else if (kcap == 16) rc = tc_launch_fold<1, 16>(has_fold, mq_hi, mq_lo, md_hi, md_lo, p, pl.grid, st);
-    else rc = tc_launch_fold<1, 32>(has_fold, mq_hi, mq_lo, md_hi, md_lo, p, pl.grid, st);
-  }
-  tc_ev_record(1, st);
-  if (rc != EMR2A_OK) return rc;
-  if (partials) {
-    partials->parts = p.keys_out;
-    partials->splits = pl.splits;
-    partials->tau = p.tau;
-    return EMR2A_OK;
-  }
-  if (pl.splits > 1)
-    return emr2a_topk_merge(reinterpret_cast<const uint64_t*>(ws + keys_off), pl.splits, Q, K, Q * K, K, K, out_keys, st);
-  return EMR2A_OK;
-}
-
-void tc_timing_record(int which, cudaStream_t st) { tc_ev_record(which, st); }
-
-int tc2_range_dispatch(bool has_fold, const CUtensorMap& a, const CUtensorMap& b, const CUtensorMap& c,
-                       const CUtensorMap& d, const TcParams& p, int grid, cudaStream_t st);
-
-// Filter of emr2a_range_search: the 1-pass (hi plane) tensor-core GEMM of tc_topk_search with the range epilogue --
-// every admissible pair with s~ >= t - E goes to cand [cand_cap] as (query, key); *count (zeroed by the caller) counts
-// them all.  Workspace: tc_topk_workspace_bytes(Q, N, 1, D) (fold padding and cohort counters of the same plan).
-// tri (emr2a_self_join): query and database rows are the rows [q_row0, ...) and [idx_base, ...) of ONE row set, only
-// pairs of global rows i < j are computed, and the query field of a candidate is the global row i.  The cohort pacing
-// of a self-join band runs when the workspace holds its counters (emr2a_self_join_workspace_bytes sizes them for the
-// whole cohort as one band; pacing never changes a result).
-int tc_range_filter(const uint16_t* q_hi, const uint16_t* db_hi, int64_t Q, int64_t N, int D, int64_t ldq, int64_t lddb,
-                    const uint8_t* q_fold, const uint8_t* db_fold, int fold_sorted, int64_t idx_base, float min_score,
-                    const float* q_stats, const float* db_stats, uint64_t* cand, int64_t cand_cap,
-                    unsigned long long* count, void* workspace, size_t ws_bytes, cudaStream_t st, bool tri,
-                    int64_t q_row0) {
-  const char* who = tri ? "self_join" : "range_search";
-  int rc = check_planes(who, q_hi, nullptr, db_hi, nullptr, Q, N, D, ldq, lddb, idx_base, 1);
-  if (rc != EMR2A_OK) return rc;
-  const int64_t Dp = (static_cast<int64_t>(D) + T_BK - 1) / T_BK * T_BK;
-  const bool has_fold = q_fold != nullptr;
-  const bool pairs = use_cta_pairs(Q);
-  const TcPlan pl = tc_plan(Q, N, 1, has_fold, pairs, 1, lddb > ldq ? lddb : ldq, 1);
-  const size_t sync_off = (pl.fold_bytes + 255) & ~static_cast<size_t>(255);
-  const size_t need = tri ? sync_off : sync_off + pl.sync_bytes;
-  if (!workspace || ws_bytes < need) return fail(EMR2A_ERR_WORKSPACE, "%s: workspace %zu < %zu", who, ws_bytes, need);
-  const bool paced = pairs && pl.sync_bytes && ws_bytes >= sync_off + pl.sync_bytes;
-  uint8_t* ws = static_cast<uint8_t*>(workspace);
-  CUtensorMap mq, md;
-  if ((rc = make_plane_map(&mq, q_hi, Q, Dp, ldq, T_BM)) != EMR2A_OK) return rc;
-  if ((rc = make_plane_map(&md, db_hi, N, Dp, lddb, pairs ? T_BN / 2 : T_BN)) != EMR2A_OK) return rc;
-  TcParams p{};
-  p.Q = Q; p.N = N; p.k_chunks = static_cast<int>(Dp / T_BK);
-  p.m_tiles = pl.m_tiles; p.n_tiles = pl.n_tiles; p.splits = pl.splits; p.tiles_per_split = pl.tiles_per_split;
-  p.idx_base = idx_base; p.K = 1;
-  p.mg = pl.mg;
-  if (paced) {
+  if (pairs && pl.sync_bytes && ws_bytes >= sync_off + pl.sync_bytes) {
     p.sync_tiles = pl.sync_tiles; p.sync_points = pl.sync_points; p.sync_budget = pl.sync_budget;
     p.sync_ctr = reinterpret_cast<uint32_t*>(ws + sync_off);
     EMR2A_CUDA_TRY(cudaMemsetAsync(p.sync_ctr, 0, pl.sync_bytes, st));
@@ -576,19 +481,90 @@ int tc_range_filter(const uint16_t* q_hi, const uint16_t* db_hi, int64_t Q, int6
     for (int i = 0; i < 8; ++i) g_last_plan[i] = plan[i];
   }
   if (has_fold) {
-    EMR2A_CUDA_TRY(cudaMemsetAsync(ws, 0xFF, pl.fold_bytes, st));
-    EMR2A_CUDA_TRY(cudaMemcpyAsync(ws, db_fold, static_cast<size_t>(N), cudaMemcpyDeviceToDevice, st));
-    p.q_fold = q_fold; p.db_fold = ws; p.fold_sorted = fold_sorted;
+    uint8_t* fpad = ws + fold_off;
+    EMR2A_CUDA_TRY(cudaMemsetAsync(fpad, 0xFF, pl.fold_bytes, st));
+    EMR2A_CUDA_TRY(cudaMemcpyAsync(fpad, db_fold, static_cast<size_t>(N), cudaMemcpyDeviceToDevice, st));
+    p.q_fold = q_fold; p.db_fold = fpad; p.fold_sorted = fold_sorted;
   }
+  return EMR2A_OK;
+}
+
+template <int P, int KC, bool R> struct Tc1 {
+  static TcKernel get(bool fold) { return fold ? tc_topk_kernel<P, KC, true, R> : tc_topk_kernel<P, KC, false, R>; }
+};
+
+// The instantiation for (passes, kcap, fold, range) (tc_pick), null if there is none; *smem = its dynamic shared memory.
+static TcKernel tc_kernel(int passes, int kcap, bool fold, bool range, size_t* smem) {
+  const int planes = passes == 3 ? 2 : 1, stages = passes == 3 ? 2 : 4;      // PLANES and STAGES of tc_topk_kernel
+  *smem = static_cast<size_t>(stages) * planes * (T_A_BYTES + T_B_BYTES) + 1024;
+  return tc_pick<Tc1>(passes, kcap, fold, range);
+}
+
+// Launches what tc_setup prepared on the kernel it planned (CTA pairs or single CTAs), between the timing events.
+static int tc_launch(const TcLaunch& L, int passes, int kcap, bool range, cudaStream_t st) {
+  size_t smem = 0;
+  const TcKernel kern = (L.pairs ? tc2_kernel : tc_kernel)(passes, kcap, L.p.q_fold != nullptr, range, &smem);
+  auto launch = [&]() -> int {
+    if (!kern) return fail(EMR2A_ERR_INVALID, "tc_launch: unsupported (passes=%d, kcap=%d, range=%d)", passes, kcap, range ? 1 : 0);
+    EMR2A_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    kern<<<L.pl.grid, T_THREADS, smem, st>>>(L.mq_hi, L.mq_lo, L.md_hi, L.md_lo, L.p);
+    EMR2A_LAUNCH_CHECK(L.pairs ? "tc2_topk_kernel" : "tc_topk_kernel");
+    return EMR2A_OK;
+  };
+  tc_ev_record(0, st);
+  const int rc = launch();
+  tc_ev_record(1, st);
+  return rc;
+}
+
+int tc_topk_search(const uint16_t* q_hi, const uint16_t* q_lo, const uint16_t* db_hi, const uint16_t* db_lo,
+                   int64_t Q, int64_t N, int D, int64_t ldq, int64_t lddb,
+                   const uint8_t* q_fold, const uint8_t* db_fold, int64_t idx_base, int K, int passes,
+                   uint64_t* out_keys, void* workspace, size_t ws_bytes, float* debug_scores, cudaStream_t st,
+                   TcPartials* partials, int fold_sorted, int min_splits) {
+  if (K > 32) return fail(EMR2A_ERR_UNSUPPORTED, "topk_search(bf16): K=%d > 32 (use EMR2A_PREC_FP32)", K);
+  TcLaunch L;
+  int rc = tc_setup(L, "topk_search(bf16)", q_hi, q_lo, db_hi, db_lo, Q, N, D, ldq, lddb, q_fold, db_fold, fold_sorted,
+                    idx_base, K, passes, min_splits, true, true, workspace, ws_bytes, st);
+  if (rc != EMR2A_OK) return rc;
+  const int splits = L.pl.splits;
+  L.p.keys_out = (splits > 1 || partials) ? L.keys : out_keys;
+  L.p.debug_scores = debug_scores;
+  rc = tc_launch(L, passes, K <= 8 ? 8 : (K <= 16 ? 16 : 32), false, st);
+  if (rc != EMR2A_OK) return rc;
+  if (partials) {
+    partials->parts = L.p.keys_out;
+    partials->splits = splits;
+    partials->tau = L.p.tau;
+    return EMR2A_OK;
+  }
+  if (splits > 1) return emr2a_topk_merge(L.keys, splits, Q, K, Q * K, K, K, out_keys, st);
+  return EMR2A_OK;
+}
+
+void tc_timing_record(int which, cudaStream_t st) { tc_ev_record(which, st); }
+
+// Filter of emr2a_range_search: the 1-pass (hi plane) tensor-core GEMM of tc_topk_search with the range epilogue --
+// every admissible pair with s~ >= t - E goes to cand [cand_cap] as (query, key); *count (zeroed by the caller) counts
+// them all.  Workspace: tc_topk_workspace_bytes(Q, N, 1, D) (fold padding and cohort counters of the same plan).
+// tri (emr2a_self_join): query and database rows are the rows [q_row0, ...) and [idx_base, ...) of ONE row set, only
+// pairs of global rows i < j are computed, and the query field of a candidate is the global row i.  The cohort pacing
+// of a self-join band runs when the workspace holds its counters (emr2a_self_join_workspace_bytes sizes them for the
+// whole cohort as one band; pacing never changes a result).
+int tc_range_filter(const uint16_t* q_hi, const uint16_t* db_hi, int64_t Q, int64_t N, int D, int64_t ldq, int64_t lddb,
+                    const uint8_t* q_fold, const uint8_t* db_fold, int fold_sorted, int64_t idx_base, float min_score,
+                    const float* q_stats, const float* db_stats, uint64_t* cand, int64_t cand_cap,
+                    unsigned long long* count, void* workspace, size_t ws_bytes, cudaStream_t st, bool tri,
+                    int64_t q_row0) {
+  TcLaunch L;
+  const int rc = tc_setup(L, tri ? "self_join" : "range_search", q_hi, nullptr, db_hi, nullptr, Q, N, D, ldq, lddb, q_fold,
+                          db_fold, fold_sorted, idx_base, 1, 1, 1, false, !tri, workspace, ws_bytes, st);
+  if (rc != EMR2A_OK) return rc;
+  TcParams& p = L.p;
   p.range_t = min_score; p.D = D; p.q_stats = q_stats; p.db_stats = db_stats;
   p.range_out = reinterpret_cast<ulonglong2*>(cand); p.range_cap = cand_cap; p.range_count = count;
   if (tri) { p.self_join = 1; p.q_row0 = q_row0; p.db_row0 = idx_base; }
-  tc_ev_record(0, st);
-  if (pairs) rc = tc2_range_dispatch(has_fold, mq, mq, md, md, p, pl.grid, st);
-  else rc = has_fold ? tc_launch<1, 8, true, true>(mq, mq, md, md, p, pl.grid, st)
-                     : tc_launch<1, 8, false, true>(mq, mq, md, md, p, pl.grid, st);
-  tc_ev_record(1, st);
-  return rc;
+  return tc_launch(L, 1, 8, true, st);
 }
 
 }  // namespace emr2a

@@ -243,35 +243,15 @@ tc2_topk_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_consta
   }
 }
 
-template <int PASSES, int KCAP, bool HAS_FOLD, bool RANGE = false>
-static int tc2_launch(const CUtensorMap& mq_hi, const CUtensorMap& mq_lo, const CUtensorMap& md_hi, const CUtensorMap& md_lo,
-                      const TcParams& p, int grid, cudaStream_t st) {
-  constexpr int PLANES = PASSES == 3 ? 2 : 1;
-  constexpr int STAGES = PASSES == 3 ? 3 : 6;
-  const size_t smem = static_cast<size_t>(STAGES) * PLANES * (T_A_BYTES + T2_BH_BYTES) + 1024;
-  auto kern = tc2_topk_kernel<PASSES, KCAP, HAS_FOLD, RANGE>;
-  EMR2A_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-  kern<<<grid, T_THREADS, smem, st>>>(mq_hi, mq_lo, md_hi, md_lo, p);
-  EMR2A_LAUNCH_CHECK("tc2_topk_kernel");
-  return EMR2A_OK;
-}
+template <int P, int KC, bool R> struct Tc2 {
+  static TcKernel get(bool fold) { return fold ? tc2_topk_kernel<P, KC, true, R> : tc2_topk_kernel<P, KC, false, R>; }
+};
 
-// dispatch over (passes, kcap, fold)
-int tc2_dispatch(int passes, int kcap, bool has_fold, const CUtensorMap& a, const CUtensorMap& b, const CUtensorMap& c,
-                 const CUtensorMap& d, const TcParams& p, int grid, cudaStream_t st) {
-#define EMR2A_TC2_CASE(P, KC)                                                                  \
-  if (passes == P && kcap == KC)                                                              \
-    return has_fold ? tc2_launch<P, KC, true>(a, b, c, d, p, grid, st) : tc2_launch<P, KC, false>(a, b, c, d, p, grid, st);
-  EMR2A_TC2_CASE(1, 8) EMR2A_TC2_CASE(1, 16) EMR2A_TC2_CASE(1, 32)
-  EMR2A_TC2_CASE(3, 8) EMR2A_TC2_CASE(3, 16) EMR2A_TC2_CASE(3, 32)
-#undef EMR2A_TC2_CASE
-  return fail(EMR2A_ERR_INVALID, "tc2_dispatch: unsupported (passes=%d, kcap=%d)", passes, kcap);
-}
-
-// range epilogue (emr2a_range_search): the 1-pass filter, no register list
-int tc2_range_dispatch(bool has_fold, const CUtensorMap& a, const CUtensorMap& b, const CUtensorMap& c,
-                       const CUtensorMap& d, const TcParams& p, int grid, cudaStream_t st) {
-  return has_fold ? tc2_launch<1, 8, true, true>(a, b, c, d, p, grid, st) : tc2_launch<1, 8, false, true>(a, b, c, d, p, grid, st);
+// The instantiation for (passes, kcap, fold, range) (tc_pick), null if there is none; *smem = its dynamic shared memory.
+TcKernel tc2_kernel(int passes, int kcap, bool fold, bool range, size_t* smem) {
+  const int planes = passes == 3 ? 2 : 1, stages = passes == 3 ? 3 : 6;      // PLANES and STAGES of tc2_topk_kernel
+  *smem = static_cast<size_t>(stages) * planes * (T_A_BYTES + T2_BH_BYTES) + 1024;
+  return tc_pick<Tc2>(passes, kcap, fold, range);
 }
 
 }  // namespace emr2a
